@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the forward hot path on B200, one BASELINE.json config per --workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -22,6 +22,11 @@ collective; one all-gather of the [B, classes] logits per step.  Prints ONE JSON
   cpu_baseline  the reference's own CPU forward on the host cores (oracle/_ref = the byte-compiled reference), bounded sample
 
 ``--impl reference`` times the reference's CPU fp32 forward itself (rank 0 only) on a bounded sample of the same workload.
+
+``--dump-outputs DIR`` writes, after the timed steps, what the last timed step returned for every GPU workload of the line as
+float32 ``DIR/<workload>_logits.npy`` / ``DIR/biggan256_images.npy`` (rank 0; logits gathered over ranks).  An output of more
+than DUMP_ELEMS elements is stored as a fixed seeded sample of that many elements (1-D, same positions every run).  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -58,6 +63,17 @@ WORKLOADS = {
                 check_clips=1, cpu_sample=2, act_elems=8 * 22.2e6),
 }
 DEFAULT_WORKLOAD = "resnet3d50"
+DUMP_ELEMS = 1 << 22        # 16 MB of float32 per array: the default line's four outputs stay within 64 MB
+
+
+def dump_array(t):
+    """``t`` as a float32 NumPy array; above DUMP_ELEMS elements, a sample of DUMP_ELEMS of them at fixed seeded positions."""
+    import torch
+    t = t.detach()
+    if t.numel() > DUMP_ELEMS:
+        idx = torch.randint(0, t.numel(), (DUMP_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.float().cpu().numpy()
 
 
 def load_peaks():
@@ -253,10 +269,11 @@ def run_reference_arm(args, spec, rank):
 # ------------------------------------------------------------------------------------------------
 # GPU arm, video / image classifiers
 # ------------------------------------------------------------------------------------------------
-def run_ours(args, spec, rank, world, local, secondary=False):
+def run_ours(args, spec, rank, world, local, secondary=False, outputs=None):
     """All GPU work of one classifier workload.  Returns the JSON line (rank 0; None elsewhere) WITHOUT its cpu_baseline: the CPU
     legs run in main() after the process group is gone, so that no rank sits in an NCCL barrier while rank 0 times the host.
-    ``secondary``: a compact measurement riding on the default line (no fp16 / uint8 e2e variants, no nested workloads)."""
+    ``secondary``: a compact measurement riding on the default line (no fp16 / uint8 e2e variants, no nested workloads).
+    ``outputs``: a dict that receives the logits of the last timed step (``dump_array``) on every rank."""
     import torch
     import torch.distributed as dist
     from pretorched_x_b200 import ops, parallel, _lib, engine
@@ -347,6 +364,8 @@ def run_ours(args, spec, rank, world, local, secondary=False):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_total = float(t.item())
     value = total * args.steps / (ms_total / 1e3)
+    if outputs is not None:
+        outputs[args.workload + "_logits"] = dump_array(parallel.gather_logits(out, total))
 
     # ---- end to end through the public API (pretorched_x_b200.graph.PipelinedForward): pinned HOST clips -> H2D -> forward ->
     #      D2H logits every step; the copy of batch i+1 overlaps the forward of batch i ----
@@ -398,16 +417,15 @@ def run_ours(args, spec, rank, world, local, secondary=False):
     if args.workload == DEFAULT_WORKLOAD and not secondary:
         del host_in
         x_keep = x_dev
-        sub_steps = max(5, min(args.steps, 20))
         todo = ([] if args.no_biggan else ["biggan256"]) + ([] if args.no_others else ["r2plus1d34", "nonlocal50"])
         for name in todo:
             torch.cuda.empty_cache()
             try:
                 if name == "biggan256":
-                    others[name] = run_biggan(args, rank, world, local, emit=False, steps=sub_steps)
+                    others[name] = run_biggan(args, rank, world, local, outputs=outputs)
                 else:
-                    sub = argparse.Namespace(**dict(vars(args), workload=name, batch=0, steps=sub_steps, layers=False))
-                    others[name] = run_ours(sub, WORKLOADS[name], rank, world, local, secondary=True)
+                    sub = argparse.Namespace(**dict(vars(args), workload=name, batch=0, layers=False))
+                    others[name] = run_ours(sub, WORKLOADS[name], rank, world, local, secondary=True, outputs=outputs)
             except Exception as exc:      # the contract's line must survive a failure of a secondary workload
                 others[name] = {"error": "%s: %s" % (type(exc).__name__, exc)}
                 print("secondary %s measurement failed: %s" % (name, others[name]["error"]), file=sys.stderr)
@@ -551,7 +569,7 @@ def run_biggan_reference_arm(args, rank):
         "gpu_launches": 0}), flush=True)
 
 
-def run_biggan(args, rank, world, local, emit=True, steps=None):
+def run_biggan(args, rank, world, local, outputs=None):
     import torch
     import torch.distributed as dist
     import pretorched_x_b200 as P
@@ -561,7 +579,7 @@ def run_biggan(args, rank, world, local, emit=True, steps=None):
 
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    steps = steps or args.steps
+    steps = args.steps
     B = args.batch if args.batch else BIGGAN_BATCH
     # random-init generator with calibrated standing statistics (a tiny CPU pass of the restatement: O(1) activations)
     model, sd_cpu, _, _ = OB.build_case(P.biggan_deep, BIGGAN_RES, BIGGAN_CH, BIGGAN_CLASSES, 4, init="ortho")
@@ -626,6 +644,8 @@ def run_biggan(args, rank, world, local, emit=True, steps=None):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_total = float(t.item())
     value = B * world * steps / (ms_total / 1e3)
+    if outputs is not None:
+        outputs["biggan256_images"] = dump_array(graphed.static_out)
     del graphed
     torch.cuda.empty_cache()
 
@@ -760,7 +780,11 @@ def main():
     ap.add_argument("--no-others", action="store_true", help="skip the secondary r2plus1d34 / nonlocal50 measurements of the default line")
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=list(WORKLOADS) + ["biggan256"],
                     help="which BASELINE.json config to time (default resnet3d50 = configs[1], the contract's line)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of every GPU workload to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -779,16 +803,22 @@ def main():
             os.environ["NCCL_DEBUG"] = "WARN"
         from pretorched_x_b200 import parallel
         parallel.init_from_env(backend="nccl")
+    outputs = {} if args.dump_outputs else None
     if args.workload == "biggan256":
-        line = run_biggan(args, rank, world, local)
+        line = run_biggan(args, rank, world, local, outputs=outputs)
     else:
-        line = run_ours(args, spec, rank, world, local)
+        line = run_ours(args, spec, rank, world, local, outputs=outputs)
     if world > 1:
         import torch.distributed as dist
         dist.barrier()
         dist.destroy_process_group()          # every rank but 0 is done: nobody spins on a GPU while the host legs run
     if rank != 0 or line is None:
         return
+    if outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if not args.no_cpu:
         def cpu_of(name, steps):
             cb = biggan_cpu(steps=steps, warmup=1) if name == "biggan256" else time_cpu(WORKLOADS[name], steps=steps, warmup=1)

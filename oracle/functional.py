@@ -15,6 +15,7 @@ the unmodified reference from /root/reference, checks these functions against it
 and stores the reference's outputs under ``tests/golden/``.  ``tests/test_oracle_golden.py`` re-checks the
 restatement against those fixtures wherever the test-suite runs.
 """
+import hashlib
 import itertools
 
 import numpy as np
@@ -468,6 +469,13 @@ def digests_match(a, b, rtol=1e-9):
             if abs(u - v) > rtol * max(abs(u), abs(v), 1e-30):
                 return False
     return True
+
+
+def state_hashes(sd):
+    """Per-tensor (shape, dtype, SHA-256 of the raw bytes): equal hashes mean ``torch.equal`` tensors, so a stored copy
+    can stand in for a state_dict that is too large to keep."""
+    return {k: (tuple(v.shape), str(v.dtype), hashlib.sha256(v.detach().contiguous().cpu().numpy().tobytes()).hexdigest())
+            for k, v in sd.items()}
 
 
 def calibrate_nonlocal_(model, x, target_std=3.0):

@@ -358,9 +358,33 @@ def run_slowfast_cases():
         print("%-32s logits %s absmax %.4f" % (name, tuple(y.shape), y.abs().max()))
 
 
+# (arch, factory kwargs, seed): whole-model inits whose every tensor tests/test_oracle_golden.py checks against the reference
+STATE_CASES = [
+    ("r2plus1d18", dict(num_classes=400), 3), ("resnet3d50", dict(num_classes=400), 3), ("nonlocalresnet3d50", dict(), 3),
+    ("resnext3d50", dict(num_classes=400), 5), ("resnext3d18", dict(num_classes=10, shortcut_type="A"), 5), ("resnext3d101", dict(), 5),
+]
+
+
+def run_state_cases():
+    """The reference's whole state_dict for each STATE_CASES init, stored as per-tensor hashes (oracle.functional.state_hashes):
+    the tensors themselves run to hundreds of MB, the hashes let a test demand bit-identical tensors without them."""
+    import warnings
+    RL.load()
+    RL.load_r2plus1d()
+    cases = []
+    for arch, kwargs, seed in STATE_CASES:
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            torch.manual_seed(seed)
+            ref = RL.build(arch, **kwargs)
+        cases.append(dict(arch=arch, kwargs=kwargs, seed=seed, tensors=OF.state_hashes(ref.state_dict())))
+        print("%-32s %d tensors" % ("state %s" % arch, len(cases[-1]["tensors"])))
+    torch.save(dict(kind="state", cases=cases, torch_version=torch.__version__), os.path.join(GOLDEN_DIR, "state_hashes.pt"))
+
+
 def main(argv=None):
     """``python -m oracle.make_golden`` regenerates everything; ``... name [name ...]`` only the named model / nlblock cases
-    or groups (``relations``, ``slowfast``, ``nlblocks``, ``resnext``, ``image``, ``preact``, ``trn``)."""
+    or groups (``relations``, ``slowfast``, ``nlblocks``, ``resnext``, ``image``, ``preact``, ``trn``, ``state``)."""
     argv = list(sys.argv[1:] if argv is None else argv)
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     torch.set_num_threads(max(1, os.cpu_count() or 1))
@@ -382,6 +406,8 @@ def main(argv=None):
         run_trn_cases()
     if want("image"):
         run_image_case()
+    if want("state"):
+        run_state_cases()
 
 
 if __name__ == "__main__":

@@ -35,6 +35,22 @@ def test_library_exports_every_declared_symbol():
     assert lib.b2_version() == _lib.EXPECTED_ABI == 103
 
 
+def test_build_digest_covers_every_included_file():
+    """The library is rebuilt only when the digest of SOURCES + HEADERS changes: a local header left out of HEADERS would let an
+    edited kernel run from a stale library."""
+    from pretorched_x_b200.csrc import build
+    listed = {os.path.normpath(os.path.join(build.HERE, f)) for f in build.SOURCES + build.HEADERS}
+    todo, seen = list(listed), set()
+    while todo:
+        path = todo.pop()
+        if path in seen:
+            continue
+        seen.add(path)
+        for inc in re.findall(r'^\s*#\s*include\s+"([^"]+)"', open(path).read(), flags=re.M):
+            todo.append(os.path.normpath(os.path.join(os.path.dirname(path), inc)))
+    assert seen <= listed, "included but not in build.HEADERS: %s" % sorted(seen - listed)
+
+
 def test_ctypes_structs_match_c_layout(tmp_path):
     prog = tmp_path / "layout.c"
     prog.write_text(
