@@ -88,6 +88,43 @@ SYMBOLS = {
 }
 
 
+# Kernel ids of the debug plan probes (enum ConvKernel in csrc/b2_conv_api.cu), one per launched template instance
+CONV_KERNELS = ("none", "tstack", "slabts", "slab<64>", "slab<128>", "slab<0>", "stem<64>", "stem<128>", "densem",
+                "pgemm<64,0>", "pgemm<64,1>", "pgemm<128,0>", "pgemm<128,1>", "igemm<64>", "igemm<128>")
+# what b2_debug_conv_plan / b2_debug_gemm_plan write: the launch, then the kernel's tiling (0 where the kernel has no such field)
+PLAN_FIELDS = ("kernel", "grid_x", "grid_y", "grid_z", "block", "smem", "cluster", "bn", "MT", "R", "PW", "WC", "wchunks", "items",
+               "flex", "remap", "groups", "tiles", "cchunks", "wbytes", "S")
+
+
+def _plan(name, argtype, args, *extra):
+    fn = getattr(load(), name)
+    fn.restype = c_int
+    fn.argtypes = [ctypes.POINTER(argtype)] + [c_int] * len(extra) + [ctypes.POINTER(c_int), c_int]
+    out = (c_int * len(PLAN_FIELDS))()
+    check(fn(ctypes.byref(args), *extra, out, len(PLAN_FIELDS)), name)
+    plan = dict(zip(PLAN_FIELDS, out))
+    plan["kernel"] = CONV_KERNELS[plan["kernel"]]
+    return plan
+
+
+def conv_plan(args):
+    """What b2_conv_ndhwc_fprop would launch for ``args`` (a ConvArgs), as a dict of PLAN_FIELDS.  Host code only: without a
+    device the library plans for 148 SMs, the B200's count."""
+    return _plan("b2_debug_conv_plan", ConvArgs, args)
+
+
+def gemm_plan(args, k2=0):
+    """What b2_gemm_f16 (k2 == 0) or b2_gemm2_f16 (a second operand pair of depth k2) would launch for ``args`` (a GemmArgs)."""
+    return _plan("b2_debug_gemm_plan", GemmArgs, args, k2)
+
+
+def last_conv_kernel():
+    """The kernel the last b2_conv_ndhwc_fprop call launched (a CONV_KERNELS name)."""
+    lib = load()
+    lib.b2_debug_last_conv_kernel.restype = c_int
+    return CONV_KERNELS[lib.b2_debug_last_conv_kernel()]
+
+
 def lib_path():
     return _LIB_PATH
 

@@ -1,7 +1,5 @@
-// b2_conv_api.cu -- C-ABI entry points for the tcgen05 implicit-GEMM convolution and the dense GEMM,
-// plus library-wide error/launch bookkeeping and the CUtensorMap builder.
-#include <atomic>
-#include <mutex>
+// b2_conv_api.cu -- C-ABI entry points for the tcgen05 convolution and dense GEMM kernels.  A host-only planner decides which
+// kernel runs a call and with what tiling (plan_conv / plan_gemm: a ConvPlan, no CUDA call but sm_count()); launch_plan runs it.
 #include <stdlib.h>
 #include <string.h>
 
@@ -17,120 +15,73 @@
 namespace b2 {
 
 // ------------------------------------------------------------------------------------------
-// error + launch bookkeeping
+// kernel-selection knobs (debug / tuning): read from the environment once, changed by the b2_debug_set_* entry points
 // ------------------------------------------------------------------------------------------
-static thread_local char g_err[512] = "";
-static std::atomic<uint64_t> g_launches{0};
+struct Tuning {
+  int conv_algo = 0;       // 0 auto, 1 gather kernel for every convolution the stem / dense-M kernels do not take (A/B comparisons)
+  int gemm_algo = 0;       // 0 auto (persistent kernel where it applies), 1 force the per-tile kernel
+  int tstack = -1;         // temporal stack kernel: -1 rule, 0 never (B2_TSTACK=0), 1 whenever the shape is eligible
+  bool slabts = true;      // temporal-group slab kernel (B2_SLABTS=0 disables)
+  int slab_mt = 0;         // M tiles per slab work item: 0 cost model, > 0 forced (B2_SLAB_MT)
+  bool slab_mp = true;     // multi-plane slab work items (B2_SLAB_MP=0 disables)
+  int slab_wide = -1;      // 256-column N tiles for channel counts that are multiples of 256: -1 rule, 0 never, 1 always
+  int densem_maxm = -1;    // dense-M kernel: -1 rule, 0 never, > 0 replaces both M thresholds (B2_DENSEM_MAXM)
+  int densem_s = 0;        // > 0 caps the dense-M cluster size (B2_DENSEM_S)
+  bool stem_pair = true;   // pair-of-planes items of the stem kernel (B2_STEM_PAIR=0 disables)
+};
 
-int set_error(int code, const char* fmt, ...) {
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(g_err, sizeof(g_err), fmt, ap);
-  va_end(ap);
-  return code;
+static bool env_off(const char* name) { const char* e = getenv(name); return e && e[0] == '0'; }
+static int env_int(const char* name, int absent) { const char* e = getenv(name); return e ? atoi(e) : absent; }
+static Tuning& tuning() {
+  static Tuning t{0, 0, env_off("B2_TSTACK") ? 0 : -1, !env_off("B2_SLABTS"), env_int("B2_SLAB_MT", 0) > 0 ? env_int("B2_SLAB_MT", 0) : 0,
+                  !env_off("B2_SLAB_MP"), -1, env_int("B2_DENSEM_MAXM", -1) >= 0 ? env_int("B2_DENSEM_MAXM", -1) : -1,
+                  env_int("B2_DENSEM_S", 0), !env_off("B2_STEM_PAIR")};
+  return t;
 }
-void count_launch(int n) { g_launches.fetch_add(static_cast<uint64_t>(n), std::memory_order_relaxed); }
 
-int require_sm100() {
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return set_error(B2_ERR_CUDA, "no CUDA device: %s", cudaGetErrorString(e));
-  int major = 0;
-  e = cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev);
-  if (e != cudaSuccess) return set_error(B2_ERR_CUDA, "cudaDeviceGetAttribute: %s", cudaGetErrorString(e));
-  if (major != 10)
-    return set_error(B2_ERR_UNSUPPORTED, "this library targets sm_100a (B200); device is sm_%d0 and there is no fallback",
-                     major);
+// ------------------------------------------------------------------------------------------
+// the plan: one launch of one kernel instance, as plain values
+// ------------------------------------------------------------------------------------------
+enum ConvKernel {          // one value per launched template instance; _lib.CONV_KERNELS names them in this order
+  KERN_NONE = 0, KERN_TSTACK, KERN_SLABTS, KERN_SLAB64, KERN_SLAB128, KERN_SLABN, KERN_STEM64, KERN_STEM128, KERN_DENSEM,
+  KERN_PGEMM64, KERN_PGEMM64_GAN, KERN_PGEMM128, KERN_PGEMM128_GAN, KERN_IGEMM64, KERN_IGEMM128
+};
+static const char* const kKernelName[] = {"none", "tstack_kernel", "slabts_kernel", "slabconv_kernel", "slabconv_kernel",
+                                          "slabconv_kernel", "stemconv_kernel", "stemconv_kernel", "densem_kernel", "pgemm_kernel",
+                                          "pgemm_kernel", "pgemm_kernel", "pgemm_kernel", "igemm_kernel", "igemm_kernel"};
+
+static const int kNumTmaps[] = {0, 2, 2, 2, 2, 2, 1, 1, 2, 7, 7, 7, 7, 4, 4};
+constexpr int kMaxTmaps = 7;
+struct ConvPlan {
+  int kernel;                       // ConvKernel
+  dim3 grid, block;
+  int smem;                         // dynamic shared memory bytes
+  int cluster;                      // CTAs per thread-block cluster along z (dense-M split-K); 1: plain launch
+  TmapSpec tm[kMaxTmaps];           // the kernel's tensor maps, in argument order (kNumTmaps[kernel] of them)
+  signed char tm_copy[kMaxTmaps];   // >= 0: the same map as tm[tm_copy[i]] (an operand the kernel does not read)
+  union {
+    SlabParams slab;                // slab kernels and the temporal-group slab kernel
+    TstackParams tstack;
+    StemParams stem;
+    DensemParams densem;
+    IgemmParams igemm;
+    PgemmParams pgemm;
+  } p;
+};
+
+static int set_launch(ConvPlan* pl, int kernel, dim3 grid, int block, int smem, int cluster = 1) {
+  pl->kernel = kernel; pl->grid = grid; pl->block = dim3(block); pl->smem = smem; pl->cluster = cluster;
   return B2_OK;
 }
-
-int current_device() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  return dev;
-}
-
-int sm_count() {               // per device ordinal (a process may drive several GPUs)
-  static std::atomic<int> cache[64];
-  const int dev = current_device() & 63;
-  int n = cache[dev].load(std::memory_order_relaxed);
-  if (n == 0) {
-    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
-    cache[dev].store(n, std::memory_order_relaxed);
-  }
-  return n;
-}
+static dim3 persistent_grid(long long work) { return dim3((unsigned)(work < sm_count() ? work : sm_count())); }   // min(work, SMs)
 
 // ------------------------------------------------------------------------------------------
-// tensor maps
+// slab convolution (stride 1 / 2, "same" padding): geometry and tiling
 // ------------------------------------------------------------------------------------------
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static PFN_encodeTiled get_encode_tiled() {
-  static PFN_encodeTiled fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<PFN_encodeTiled>(p);
-  });
-  return fn;
-}
-
-int make_tmap_2d_f16(CUtensorMap* out, const void* base, uint64_t inner, uint64_t outer, uint64_t pitch_elems,
-                     uint32_t box_inner, uint32_t box_outer, bool swizzle128) {
-  PFN_encodeTiled enc = get_encode_tiled();
-  if (!enc) return set_error(B2_ERR_CUDA, "cuTensorMapEncodeTiled entry point unavailable (no driver?)");
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return set_error(B2_ERR_INVALID, "tensor base not 16-byte aligned");
-  if ((pitch_elems * 2) % 16 != 0) return set_error(B2_ERR_INVALID, "row pitch %llu elements is not a multiple of 8",
-                                                    (unsigned long long)pitch_elems);
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {pitch_elems * 2};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS)
-    return set_error(B2_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) inner=%llu outer=%llu pitch=%llu box=%ux%u", (int)r,
-                     (unsigned long long)inner, (unsigned long long)outer, (unsigned long long)pitch_elems, box_inner,
-                     box_outer);
-  return B2_OK;
-}
-
-int make_tmap_ndhwc_slab(CUtensorMap* out, const void* base, uint64_t C, uint64_t W, uint64_t H, uint64_t planes,
-                         uint32_t box_w, uint32_t box_h, uint32_t stride_hw, uint32_t box_planes) {
-  PFN_encodeTiled enc = get_encode_tiled();
-  if (!enc) return set_error(B2_ERR_CUDA, "cuTensorMapEncodeTiled entry point unavailable (no driver?)");
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return set_error(B2_ERR_INVALID, "tensor base not 16-byte aligned");
-  cuuint64_t dims[4] = {C, W, H, planes};
-  cuuint64_t strides[3] = {C * 2, W * C * 2, H * W * C * 2};
-  // with element strides the box is given in traversed (full-resolution) elements; smem receives every
-  // stride_hw-th pixel / row, i.e. box_w x box_h dense pixels
-  cuuint32_t box[4] = {64, stride_hw * (box_w - 1) + 1, stride_hw * (box_h - 1) + 1, box_planes};
-  cuuint32_t estr[4] = {1, stride_hw, stride_hw, 1};
-  if (box[1] > 256 || box[2] > 256) return set_error(B2_ERR_UNSUPPORTED, "slab box %ux%u exceeds the TMA box limit", box[1], box[2]);
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS)
-    return set_error(B2_ERR_CUDA, "cuTensorMapEncodeTiled(4d) failed (%d) C=%llu W=%llu H=%llu planes=%llu box=%ux%u", (int)r,
-                     (unsigned long long)C, (unsigned long long)W, (unsigned long long)H, (unsigned long long)planes, box_w, box_h);
-  return B2_OK;
-}
-
-// ------------------------------------------------------------------------------------------
-// slab convolution launcher (stride 1, "same" padding)
-// ------------------------------------------------------------------------------------------
-static int g_conv_algo = 0;   // 0 auto, 1 force gather (debug / A-B comparisons)
-static int g_slab_wide = -1;       // 256-column N tiles for channel counts that are multiples of 256: -1 rule below, 0 never, 1 always (tuning)
-static int g_slab_force_mt = -1;   // M tiles per slab work item: -1 read B2_SLAB_MT once, 0 cost model, > 0 forced (tuning)
-
 static int slab_naff(int ldy) { return (ldy + 31) / 32 * 32 + 256; }   // chunk reads may run past ldy inside the last N tile
+static long long slab_smem(long long slab_bytes, int w_stage, int ldy) {
+  return kSlabSStages * slab_bytes + kSlabWStages * w_stage + 256 + 2 * slab_naff(ldy) * 4 + 1024;
+}
 
 static int slab_rows(int MT, int PW, int reach, int P) {
   int R = 0;
@@ -224,16 +175,14 @@ static bool slab_geometry(const b2_conv_args* a, SlabParams* p, int wc_hint) {
   return p->n_sub > 0 && p->PW <= 256;
 }
 
-template <int BNT>   // BNT = 0: runtime N tile p.bn (set by the caller)
-static int launch_slab(const b2_conv_args* a, SlabParams& p, int MT, int R, cudaStream_t stream) {
-  if (BNT) { p.bn = BNT; p.wbytes = BNT * 128; p.accs = BNT; }
-  const int BN = p.bn;
+// Fills the run-time part of SlabParams that the slab and temporal-group kernels share; the caller sets the N tile, the
+// accumulator sets, the N tiles and the work items.
+static void slab_fill(const b2_conv_args* a, SlabParams& p, int MT, int R) {
   p.R = R;
   p.planes_total = a->N * p.To;
   p.plane_stride = R * p.PW * 128;
   p.slab_bytes = ((R * p.PW * 128 * (p.mp > 1 ? p.mp : 1)) + 1023) / 1024 * 1024;
   p.MT = MT;
-  p.nacc = (MT * p.accs <= 256) ? 2 : 1;
   p.Ncols = a->K;
   p.scale = a->scale; p.shift = a->shift;
   p.residual = reinterpret_cast<const __half*>(a->residual);
@@ -243,35 +192,20 @@ static int launch_slab(const b2_conv_args* a, SlabParams& p, int MT, int R, cuda
   p.relu = a->relu;
   p.aff_ld = a->aff_ld;
   p.naff = slab_naff(a->ldy);
-  p.tiles_n = (a->ldy + BN - 1) / BN;
   p.tiles_q = p.mp > 1 ? 1 : (p.P + MT * 128 - 1) / (MT * 128);
-  const long long plane_items = p.mp > 1 ? ((long long)a->N * p.To + p.mp - 1) / p.mp : (long long)a->N * p.To;
-  const long long items = (long long)p.tiles_n * p.tiles_q * p.wchunks * plane_items * (p.up ? 4 : 1);
-  if (items >= (1ll << 31)) return set_error(B2_ERR_INVALID, "slab problem too large");
-  p.items_total = (int)items;
-  p.fd_tiles_n = make_fastdiv(p.tiles_n); p.fd_tiles_q = make_fastdiv(p.tiles_q); p.fd_wchunks = make_fastdiv(p.wchunks);
-  p.fd_To = make_fastdiv(p.To); p.fd_PW = make_fastdiv(p.PW);
-  if (a->aff_ld && ((a->aff_ld & 3) || (reinterpret_cast<uintptr_t>(a->scale) & 15) || (reinterpret_cast<uintptr_t>(a->shift) & 15)))
-    return set_error(B2_ERR_INVALID, "per-sample scale/shift must be 16-byte aligned with a pitch that is a multiple of 4 floats");
-  const int smem_bytes = kSlabSStages * p.slab_bytes + kSlabWStages * p.wbytes + 256 + 2 * slab_naff(a->ldy) * 4 + 1024;
-  B2_OPT_IN_SMEM(slabconv_kernel<BNT>, 227 * 1024);
-  CUtensorMap tmX, tmB;
-  int rc;
-  const int taps = p.up ? 16 : a->kt * a->kh * a->kw;
-  if ((rc = make_tmap_ndhwc_slab(&tmX, a->x, (uint64_t)a->C, (uint64_t)a->W, (uint64_t)a->H, (uint64_t)a->N * a->T,
-                                 (uint32_t)p.PW, (uint32_t)R, (uint32_t)p.ss, (uint32_t)(p.mp > 1 ? p.mp : 1))) != B2_OK)
-    return rc;
-  if ((rc = make_tmap_2d_f16(&tmB, a->w, (uint64_t)taps * a->C, (uint64_t)a->K, (uint64_t)taps * a->C, 64, BN, true)) != B2_OK)
-    return rc;
-  const int grid = p.items_total < sm_count() ? p.items_total : sm_count();
-  B2_CHECK_CUDA(launch_pdl(slabconv_kernel<BNT>, dim3(grid), dim3(kSlabThreads), smem_bytes, stream, tmX, tmB, p));
-  B2_CHECK_LAUNCH("slabconv_kernel");
-  return B2_OK;
+  p.fd_tiles_q = make_fastdiv(p.tiles_q); p.fd_wchunks = make_fastdiv(p.wchunks); p.fd_PW = make_fastdiv(p.PW);
 }
 
-// Picks the N tile (fixed 64 / 128 or runtime), the M tiles per work item and the slab rows for a geometry; *best_mt == 0
-// when no configuration fits in shared memory.
-static double slab_pick_tiles(const b2_conv_args* a, SlabParams& p, int* BN_out, bool* flex_out, int* best_mt_out, int* best_R_out, bool wide = false) {
+struct SlabTiles {
+  int bn;          // N tile
+  bool flex;       // runtime-N instance (slabconv_kernel<0>)
+  int mt, R;       // M tiles per work item and slab rows; mt == 0: no configuration fits in shared memory
+  double cost;     // modelled cycles
+};
+
+// Picks the N tile (fixed 64 / 128 or runtime), the M tiles per work item and the slab rows for a geometry.
+static SlabTiles slab_pick_tiles(const b2_conv_args* a, SlabParams& p, bool wide) {
+  const Tuning& t = tuning();
   int BN = (a->ldy <= 64) ? 64 : 128;
   const int planes = a->N * p.To;
   int ntn = (a->ldy + BN - 1) / BN;
@@ -281,7 +215,7 @@ static double slab_pick_tiles(const b2_conv_args* a, SlabParams& p, int* BN_out,
   if (a->ldy > 128) {
     const int tn = (a->ldy + 255) / 256;
     const int bn = (((a->ldy + tn - 1) / tn) + 15) / 16 * 16;
-    if ((long long)bn * tn * 21 <= (long long)ntn * 128 * 20 || ((wide || g_slab_wide == 1) && a->ldy % 256 == 0)) {
+    if ((long long)bn * tn * 21 <= (long long)ntn * 128 * 20 || ((wide || t.slab_wide == 1) && a->ldy % 256 == 0)) {
       flex = true; BN = bn; ntn = tn;
       p.bn = bn; p.wbytes = (bn * 128 + 1023) / 1024 * 1024; p.accs = (bn + 31) / 32 * 32;
     }
@@ -298,17 +232,14 @@ static double slab_pick_tiles(const b2_conv_args* a, SlabParams& p, int* BN_out,
   // from ncu: a 128xNx16 MMA retires in ~40 + N/2 cycles, TMA delivers ~48 B/cycle/SM out of L2.)
   int best_mt = 0, best_R = 0;
   double best_cost = 0.0;
-  int& force_mt = g_slab_force_mt;
-  if (force_mt < 0) { const char* e = getenv("B2_SLAB_MT"); force_mt = e ? atoi(e) : 0; }   // debug / tuning only
+  const int force_mt = t.slab_mt;
   int ksteps = 0;
   for (int cc = 0; cc < p.cchunks; ++cc) { const int k = (a->C - cc * 64 + 15) / 16; ksteps += k > 4 ? 4 : k; }
   int taps_hw = 0;
   for (int sidx = 0; sidx < p.n_sub; ++sidx) taps_hw += p.sub_ntaps[sidx];
   // planes of at most one M tile whose temporal taps do not differ from plane to plane: the MT accumulators of an item are MT
   // consecutive PLANES (SlabParams::mp), see b2_slabconv.cuh
-  static int mp_env = -1;
-  if (mp_env < 0) { const char* e = getenv("B2_SLAB_MP"); mp_env = (e && e[0] == '0') ? 0 : 1; }
-  const bool mp_ok = mp_env && p.P <= 128 && (a->kt == 1 || a->T == 1) && p.ss == 1 && !p.up && p.wchunks == 1 && planes > 1 &&
+  const bool mp_ok = t.slab_mp && p.P <= 128 && (a->kt == 1 || a->T == 1) && p.ss == 1 && !p.up && p.wchunks == 1 && planes > 1 &&
                      !a->aff_ld;      // (a per-sample affine is read once per item: its tiles must belong to one image)
   p.mp = 0;
   for (int MT = 512 / acc_stride > 4 ? 4 : 512 / acc_stride; MT >= 1; --MT) {
@@ -317,8 +248,7 @@ static double slab_pick_tiles(const b2_conv_args* a, SlabParams& p, int* BN_out,
     const int R = mp_ok ? (p.P - 1 + p.reach) / p.PW + (p.reach + p.PW - 1) / p.PW + 1 : slab_rows(MT, p.PW, p.reach, p.P);
     if (p.ss * (R - 1) + 1 > 256) continue;
     const long long slab_b = ((long long)R * p.PW * 128 * (mp_ok ? MT : 1) + 1023) / 1024 * 1024;
-    const long long smem = 2ll * slab_b + kSlabWStages * w_stage + 256 + 2 * slab_naff(a->ldy) * 4 + 1024;
-    if (smem > 227 * 1024) continue;
+    if (slab_smem(slab_b, w_stage, a->ldy) > 227 * 1024) continue;
     const long long tq = mp_ok ? 1 : (p.P + MT * 128 - 1) / (MT * 128);
     const long long items = (long long)ntn * tq * (mp_ok ? (planes + MT - 1) / MT : planes) * p.wchunks * (p.up ? 4 : 1);
     const double rounds = (double)((items + sm_count() - 1) / sm_count());
@@ -333,12 +263,6 @@ static double slab_pick_tiles(const b2_conv_args* a, SlabParams& p, int* BN_out,
     const double load = (double)p.kt * p.n_sub * p.cchunks * slab_b / bpc + (double)p.kt * taps_hw * p.cchunks * w_stage / bpc;
     const double epi = (MT * acc_stride <= 256) ? 0.0 : tiles_per_item * ((BN + 31) / 32) * 250.0;
     const double cost = rounds * ((mma > load ? mma : load) + epi + 1500.0);
-    if (force_mt == -1) {                                   // previous rule (A/B): largest power-of-two MT with >= 2 rounds of items
-      if ((MT & (MT - 1)) != 0 && !flex) continue;
-      best_mt = MT; best_R = R;
-      if (items >= 2 * 148) break;
-      continue;
-    }
     if (best_mt == 0 || cost < best_cost || (force_mt > 0 && MT == force_mt)) { best_mt = MT; best_R = R; best_cost = cost; }
     if (force_mt > 0 && MT == force_mt) break;
   }
@@ -347,23 +271,21 @@ static double slab_pick_tiles(const b2_conv_args* a, SlabParams& p, int* BN_out,
     const int R4 = (p.P - 1 + p.reach) / p.PW + (p.reach + p.PW - 1) / p.PW + 1;
     const long long slab4 = ((long long)R4 * p.PW * 128 * 4 + 1023) / 1024 * 1024;
     const long long items4 = (long long)ntn * ((planes + 3) / 4);
-    if (2ll * slab4 + kSlabWStages * w_stage + 256 + 2 * slab_naff(a->ldy) * 4 + 1024 <= 227 * 1024 && items4 >= sm_count()) { best_mt = 4; best_R = R4; }
+    if (slab_smem(slab4, w_stage, a->ldy) <= 227 * 1024 && items4 >= sm_count()) { best_mt = 4; best_R = R4; }
   }
   p.mp = (mp_ok && best_mt > 1) ? best_mt : 0;
-  *BN_out = BN; *flex_out = flex; *best_mt_out = best_mt; *best_R_out = best_R;
-  return best_cost;
+  return SlabTiles{BN, flex, best_mt, best_R, best_cost};
 }
 
-// returns 1 when the slab kernel took the convolution, 0 when it does not apply, <0 on error
-static int try_slab(const b2_conv_args* a_in, cudaStream_t stream) {
-  if (g_conv_algo == 1) return 0;
-  SlabParams p;
-  b2_conv_args remap = *a_in;
+// The slab kernel.  Declines (B2_OK, no kernel) shapes it does not take.
+static int plan_slab(const b2_conv_args* a_in, ConvPlan* pl) {
+  b2_conv_args remap;
   const b2_conv_args* a = a_in;
   int wc_hint = 0;
-  if (a_in->kt > 1 && a_in->kh == 1 && a_in->kw == 1 && a_in->st == 1 && a_in->sh == 1 && a_in->sw == 1 &&
-      a_in->ph == 0 && a_in->pw == 0 && g_conv_algo != 3) {
+  if (a_in->kt > 1 && a_in->kh == 1 && a_in->kw == 1 && a_in->st == 1 && a_in->sh == 1 && a_in->sw == 1 && a_in->ph == 0 &&
+      a_in->pw == 0) {
     // (kt,1,1) over [N][T][H][W] == (1,kt,1) over N images of T rows x (H*W) columns
+    remap = *a_in;
     remap.T = 1; remap.H = a_in->T; remap.W = a_in->H * a_in->W;
     remap.kt = 1; remap.kh = a_in->kt; remap.kw = 1;
     remap.pt = 0; remap.ph = a_in->pt; remap.pw = 0;
@@ -375,170 +297,129 @@ static int try_slab(const b2_conv_args* a_in, cudaStream_t stream) {
   // per item for wide images -- with few-tap 2-D filters the per-item costs (decode, epilogue set-up, slab latency) are
   // what the cycle model trades against the extra halo columns.  The cheapest modelled configuration wins.
   const int wc_try[3] = {wc_hint, 128, 64};
-  int BN = 0, best_mt = 0, best_R = 0;
-  bool flex = false;
-  double best_cost = 0.0;
-  SlabParams best_p;
+  SlabParams& p = pl->p.slab;
+  SlabTiles best = {};
   for (int attempt = 0; attempt < 3; ++attempt) {
     if (attempt > 0 && (wc_hint > 0 || wc_try[attempt] >= a->W)) continue;
     SlabParams q;
-    if (!slab_geometry(a, &q, wc_try[attempt])) { if (attempt == 0) return 0; else continue; }
+    if (!slab_geometry(a, &q, wc_try[attempt])) { if (attempt == 0) return B2_OK; else continue; }
     if (attempt > 0 && q.wchunks == 1) continue;              // same geometry as the default
-    if (g_conv_algo == 2 && q.ss != 1) return 0;              // debug: strided convs through the gather kernel
-    int bn_c = 0, mt_c = 0, r_c = 0;
-    bool flex_c = false;
-    double cost = slab_pick_tiles(a, q, &bn_c, &flex_c, &mt_c, &r_c);
-    if (g_slab_wide < 0 && a->ldy % 256 == 0 && !flex_c) {
+    SlabTiles c = slab_pick_tiles(a, q, false);
+    if (tuning().slab_wide < 0 && a->ldy % 256 == 0 && !c.flex) {
       // 256-column N tiles (one A read per 256 output channels instead of per 128): measured with tools/conv_sweep.py
       // (profiles/slab_wide_sweep_r02.txt) they win by 5-35% wherever at least 64 work items of at least two M tiles remain, and lose
       // when halving the number of N tiles leaves SMs idle (M = 6272: 33 -> 41 us) or an item is a single tile (7x7 planes: 23 -> 29 us)
       SlabParams qw = q;
-      int bn_w = 0, mt_w = 0, r_w = 0;
-      bool flex_w = false;
-      const double cost_w = slab_pick_tiles(a, qw, &bn_w, &flex_w, &mt_w, &r_w, true);
-      if (mt_w != 0 && flex_w) {
-        const long long tq = (qw.P + mt_w * 128 - 1) / (mt_w * 128);
-        const long long items_w = (long long)((a->ldy + bn_w - 1) / bn_w) * tq * a->N * qw.To * qw.wchunks * (qw.up ? 4 : 1);
+      const SlabTiles w = slab_pick_tiles(a, qw, true);
+      if (w.mt != 0 && w.flex) {
+        const long long tq = (qw.P + w.mt * 128 - 1) / (w.mt * 128);
+        const long long items_w = (long long)((a->ldy + w.bn - 1) / w.bn) * tq * a->N * qw.To * qw.wchunks * (qw.up ? 4 : 1);
         const double tiles_per_item = (double)((qw.P + 127) / 128) / (double)tq;
-        if (items_w >= 64 && tiles_per_item >= 2.0) { q = qw; bn_c = bn_w; flex_c = flex_w; mt_c = mt_w; r_c = r_w; cost = cost_w * 0.8; }
+        if (items_w >= 64 && tiles_per_item >= 2.0) { q = qw; c = w; c.cost = w.cost * 0.8; }
       }
     }
-    if (mt_c == 0) continue;
-    if (best_mt == 0 || cost < best_cost) { best_p = q; BN = bn_c; flex = flex_c; best_mt = mt_c; best_R = r_c; best_cost = cost; }
+    if (c.mt == 0) continue;
+    if (best.mt == 0 || c.cost < best.cost) { p = q; best = c; }
   }
-  if (best_mt != 0) p = best_p;
-  if (best_mt == 0) return 0;
-  int rc = flex ? launch_slab<0>(a, p, best_mt, best_R, stream)
-                : (BN == 64) ? launch_slab<64>(a, p, best_mt, best_R, stream) : launch_slab<128>(a, p, best_mt, best_R, stream);
-  return rc == B2_OK ? 1 : rc;
+  if (best.mt == 0) return B2_OK;
+  if (!best.flex) { p.bn = best.bn; p.wbytes = best.bn * 128; p.accs = best.bn; }
+  slab_fill(a, p, best.mt, best.R);
+  p.nacc = (best.mt * p.accs <= 256) ? 2 : 1;
+  p.tiles_n = (a->ldy + p.bn - 1) / p.bn;
+  const long long plane_items = p.mp > 1 ? ((long long)a->N * p.To + p.mp - 1) / p.mp : (long long)a->N * p.To;
+  const long long items = (long long)p.tiles_n * p.tiles_q * p.wchunks * plane_items * (p.up ? 4 : 1);
+  if (items >= (1ll << 31)) return set_error(B2_ERR_INVALID, "slab problem too large");
+  p.items_total = (int)items;
+  p.fd_tiles_n = make_fastdiv(p.tiles_n); p.fd_To = make_fastdiv(p.To);
+  if (a->aff_ld && ((a->aff_ld & 3) || (reinterpret_cast<uintptr_t>(a->scale) & 15) || (reinterpret_cast<uintptr_t>(a->shift) & 15)))
+    return set_error(B2_ERR_INVALID, "per-sample scale/shift must be 16-byte aligned with a pitch that is a multiple of 4 floats");
+  const int taps = p.up ? 16 : a->kt * a->kh * a->kw;
+  B2_TRY(tmap_ndhwc_slab(&pl->tm[0], a->x, (uint64_t)a->C, (uint64_t)a->W, (uint64_t)a->H, (uint64_t)a->N * a->T, (uint32_t)p.PW,
+                         (uint32_t)p.R, (uint32_t)p.ss, (uint32_t)(p.mp > 1 ? p.mp : 1)));
+  B2_TRY(tmap_2d_f16(&pl->tm[1], a->w, (uint64_t)taps * a->C, (uint64_t)a->K, (uint64_t)taps * a->C, 64, p.bn, true));
+  return set_launch(pl, best.flex ? KERN_SLABN : best.bn == 64 ? KERN_SLAB64 : KERN_SLAB128, persistent_grid(p.items_total), kSlabThreads,
+                    (int)slab_smem(p.slab_bytes, p.wbytes, a->ldy));
 }
-
 
 // ------------------------------------------------------------------------------------------
 // temporal-group slab kernel (b2_slabts.cuh): 3 x kh x kw stride-1 "same" convolutions with <= 64 output channels
 // ------------------------------------------------------------------------------------------
-static int g_slabts = -1;     // B2_SLABTS=0 disables (A/B measurements)
-static int try_slabts(const b2_conv_args* a, cudaStream_t stream) {
-  if (g_slabts < 0) { const char* e = getenv("B2_SLABTS"); g_slabts = (e && e[0] == '0') ? 0 : 1; }
-  if (!g_slabts || g_conv_algo != 0) return 0;
-  if (a->mode != B2_CONV_AUTO || a->out_f32 || a->upsample || a->aff_ld || a->y2 || a->residual_up || a->residual_pre || a->in_scale) return 0;
-  if (a->kt != 3 || a->st != 1 || a->pt != 1 || a->sh != 1 || a->sw != 1 || a->ldy > 64 || a->T < 3) return 0;
+static int plan_slabts(const b2_conv_args* a, ConvPlan* pl) {
+  if (!tuning().slabts) return B2_OK;
+  if (a->kt != 3 || a->st != 1 || a->pt != 1 || a->sh != 1 || a->sw != 1 || a->ldy > 64 || a->T < 3) return B2_OK;
   // Measured (CUDA-graph replays, profiles/README_r02.md): 180 vs 186 us on the 3x3x3 C64->64 layer of resnet3d50 -- the operand
   // traffic it saves in shared memory comes back as 2.5x more weight bytes per output tile from L2 (one 24 KB stack per tap and input
   // frame, two M tiles per item) -- and it LOSES where the single accumulator set exposes a residual read (243 vs 190 us) or the
   // in-plane filter is 1x1 (the (3,1,1) convolutions of R(2+1)D: 64 vs 31 us against the frames-as-rows remap).  So: true 3-D
   // filters without a residual only.
-  if (a->kh * a->kw < 9 || a->residual) return 0;
-  SlabParams p;
-  if (!slab_geometry(a, &p, 0) || p.n_sub != 1) return 0;
+  if (a->kh * a->kw < 9 || a->residual) return B2_OK;
+  SlabParams& p = pl->p.slab;
+  if (!slab_geometry(a, &p, 0) || p.n_sub != 1) return B2_OK;
   int MT = p.P > 128 ? 2 : 1, R = 0;
   long long smem = 0;
   for (; MT >= 1; --MT) {
     R = slab_rows(MT, p.PW, p.reach, p.P);
-    const long long slab_b = ((long long)R * p.PW * 128 + 1023) / 1024 * 1024;
-    smem = kSlabSStages * slab_b + kSlabWStages * kTsWBytes + 256 + 2 * slab_naff(a->ldy) * 4 + 1024;
+    smem = slab_smem(((long long)R * p.PW * 128 + 1023) / 1024 * 1024, kTsWBytes, a->ldy);
     if (R <= 256 && smem <= 227 * 1024) break;
   }
-  if (MT < 1) return 0;
-  p.R = R;
-  p.planes_total = a->N * p.To;
-  p.plane_stride = R * p.PW * 128;
-  p.slab_bytes = ((R * p.PW * 128 * (p.mp > 1 ? p.mp : 1)) + 1023) / 1024 * 1024;
-  p.MT = MT; p.nacc = 1; p.bn = kTsBN; p.wbytes = kTsWBytes; p.accs = kTsBN;
-  p.Ncols = a->K;
-  p.scale = a->scale; p.shift = a->shift;
-  p.residual = reinterpret_cast<const __half*>(a->residual);
-  p.ldr = a->ldr;
-  p.y = reinterpret_cast<__half*>(a->y);
-  p.ldy = a->ldy;
-  p.relu = a->relu;
-  p.naff = slab_naff(a->ldy);
+  if (MT < 1) return B2_OK;
+  slab_fill(a, p, MT, R);
+  p.nacc = 1; p.bn = kTsBN; p.wbytes = kTsWBytes; p.accs = kTsBN;
   p.tiles_n = 1;
-  p.tiles_q = (p.P + MT * 128 - 1) / (MT * 128);
   const int groups = (p.To + kTsGroup - 1) / kTsGroup;
   const long long items = (long long)p.tiles_q * p.wchunks * a->N * groups;
-  if (items >= (1ll << 31)) return 0;
+  if (items >= (1ll << 31)) return B2_OK;
   p.items_total = (int)items;
-  p.fd_tiles_n = make_fastdiv(1); p.fd_tiles_q = make_fastdiv(p.tiles_q); p.fd_wchunks = make_fastdiv(p.wchunks);
-  p.fd_To = make_fastdiv(groups); p.fd_PW = make_fastdiv(p.PW);
-  B2_OPT_IN_SMEM(slabts_kernel, 227 * 1024);
-  CUtensorMap tmX, tmB;
-  int rc;
+  p.fd_tiles_n = make_fastdiv(1); p.fd_To = make_fastdiv(groups);
   const int taps = a->kt * a->kh * a->kw;
-  if ((rc = make_tmap_ndhwc_slab(&tmX, a->x, (uint64_t)a->C, (uint64_t)a->W, (uint64_t)a->H, (uint64_t)a->N * a->T, (uint32_t)p.PW,
-                                 (uint32_t)R, 1u)) != B2_OK) return rc;
-  if ((rc = make_tmap_2d_f16(&tmB, a->w, (uint64_t)taps * a->C, (uint64_t)a->K, (uint64_t)taps * a->C, 64, kTsBN, true)) != B2_OK) return rc;
-  const int grid = p.items_total < sm_count() ? p.items_total : sm_count();
-  B2_CHECK_CUDA(launch_pdl(slabts_kernel, dim3(grid), dim3(kSlabThreads), (size_t)smem, stream, tmX, tmB, p));
-  B2_CHECK_LAUNCH("slabts_kernel");
-  return 1;
+  B2_TRY(tmap_ndhwc_slab(&pl->tm[0], a->x, (uint64_t)a->C, (uint64_t)a->W, (uint64_t)a->H, (uint64_t)a->N * a->T, (uint32_t)p.PW,
+                         (uint32_t)R, 1u));
+  B2_TRY(tmap_2d_f16(&pl->tm[1], a->w, (uint64_t)taps * a->C, (uint64_t)a->K, (uint64_t)taps * a->C, 64, kTsBN, true));
+  return set_launch(pl, KERN_SLABTS, persistent_grid(p.items_total), kSlabThreads, (int)smem);
 }
 
 // ------------------------------------------------------------------------------------------
 // temporal stack kernel (b2_tstack.cuh): (kt,1,1) stride-1 "same" convolutions with <= 64 output channels, resident filter
 // ------------------------------------------------------------------------------------------
-static int g_last_conv_path = 0;   // which launcher took the last b2_conv_ndhwc_fprop call: 0 generic, 1 tstack (tests pin the dispatch)
-static int g_tstack = -2;     // -2: read B2_TSTACK once (0 = never); -1 rule below, 0 never, 1 whenever the shape is eligible (tests / sweeps)
-// Shape test + work decomposition (host only).  Returns false when the kernel does not take the convolution.
-static bool tstack_plan(const b2_conv_args* a, TstackParams* out, size_t* smem_out) {
-  if (a->mode != B2_CONV_AUTO || a->out_f32 || a->upsample || a->aff_ld || a->y2 || a->residual_up || a->residual_pre || a->in_scale) return false;
+static int plan_tstack(const b2_conv_args* a, ConvPlan* pl) {
+  const int mode = tuning().tstack;
+  if (mode == 0) return B2_OK;
   if (a->kh != 1 || a->kw != 1 || a->kt < 3 || !(a->kt & 1) || a->st != 1 || a->sh != 1 || a->sw != 1 || a->pt != a->kt / 2 || a->ph != 0 ||
       a->pw != 0 || a->ldy > 64 || a->T < 2)
-    return false;
+    return B2_OK;
   const int cchunks = (a->C + 63) / 64;
   const long long wbytes = (long long)cchunks * a->kt * kTkWBlock;
-  if (wbytes > 144 * 1024) return false;                     // the filter must stay resident next to the A ring
+  if (wbytes > 144 * 1024) return B2_OK;                     // the filter must stay resident next to the A ring
   const long long HW = (long long)a->H * a->W;
-  if (HW >= (1ll << 24)) return false;
-  TstackParams p;
+  if (HW >= (1ll << 24)) return B2_OK;
+  TstackParams& p = pl->p.tstack;
+  p = TstackParams{};
   p.T = a->T; p.HW = (int)HW; p.C = a->C;
   p.kt = a->kt; p.pt = a->pt;
   p.cchunks = cchunks;
   p.groups = (a->T + kTkG - 1) / kTkG;
   p.tiles_q = (int)((HW + 127) / 128);
   const long long items = (long long)a->N * p.groups * p.tiles_q;
-  if (items >= (1ll << 31)) return false;
+  if (items >= (1ll << 31)) return B2_OK;
   // Below one work item per SM the frames-as-rows form of the slab kernel (more, smaller items) keeps more SMs busy
   // (2 clips of the (3,1,1) C144 layer, 56 items: 9.6 vs 11.0 us, profiles/tstack_sweep_r02.txt).
-  if (g_tstack < 0 && items < sm_count()) return false;
+  if (mode < 0 && items < sm_count()) return B2_OK;
   p.items_total = (int)items;
   p.Ncols = a->K; p.ldy = a->ldy; p.ldr = a->ldr; p.relu = a->relu;
   p.scale = a->scale; p.shift = a->shift;
   p.residual = reinterpret_cast<const __half*>(a->residual);
   p.y = reinterpret_cast<__half*>(a->y);
   p.fd_tiles_q = make_fastdiv(p.tiles_q); p.fd_groups = make_fastdiv(p.groups);
-  *out = p;
-  *smem_out = 1024 + (size_t)kTkStages * kTkABytes + (size_t)wbytes + 128 + 512 + 64;
-  return true;
-}
-
-static int try_tstack(const b2_conv_args* a, cudaStream_t stream) {
-  if (g_tstack == -2) { const char* e = getenv("B2_TSTACK"); g_tstack = (e && e[0] == '0') ? 0 : -1; }
-  if (g_tstack == 0 || g_conv_algo != 0) return 0;
-  TstackParams p;
-  size_t smem = 0;
-  if (!tstack_plan(a, &p, &smem)) return 0;
-  const long long HW = p.HW;
-  B2_OPT_IN_SMEM(tstack_kernel, 227 * 1024);
-  CUtensorMap tmX, tmB;
-  int rc;
-  if ((rc = make_tmap_ndhwc_slab(&tmX, a->x, (uint64_t)a->C, (uint64_t)HW, 1, (uint64_t)a->N * a->T, 128u, 1u, 1u)) != B2_OK) return rc;
-  if ((rc = make_tmap_2d_f16(&tmB, a->w, (uint64_t)a->kt * a->C, (uint64_t)a->K, (uint64_t)a->kt * a->C, 64, 64, true)) != B2_OK) return rc;
-  const int grid = p.items_total < sm_count() ? p.items_total : sm_count();
-  B2_CHECK_CUDA(launch_pdl(tstack_kernel, dim3(grid), dim3(kTkThreads), smem, stream, tmX, tmB, p));
-  B2_CHECK_LAUNCH("tstack_kernel");
-  g_last_conv_path = 1;
-  return 1;
+  B2_TRY(tmap_ndhwc_slab(&pl->tm[0], a->x, (uint64_t)a->C, (uint64_t)HW, 1, (uint64_t)a->N * a->T, 128u, 1u, 1u));
+  B2_TRY(tmap_2d_f16(&pl->tm[1], a->w, (uint64_t)a->kt * a->C, (uint64_t)a->K, (uint64_t)a->kt * a->C, 64, 64, true));
+  return set_launch(pl, KERN_TSTACK, persistent_grid(p.items_total), kTkThreads, (int)(1024 + kTkStages * kTkABytes + wbytes + 128 + 512 + 64));
 }
 
 // ------------------------------------------------------------------------------------------
-// stem convolution launcher (Toeplitz-descriptor kernel)
+// stem convolution (Toeplitz-descriptor kernel)
 // ------------------------------------------------------------------------------------------
-template <int BN>
-static int launch_stem(const b2_conv_args* a, cudaStream_t stream) {
-  PFN_encodeTiled enc = get_encode_tiled();
-  if (!enc) return set_error(B2_ERR_CUDA, "cuTensorMapEncodeTiled entry point unavailable (no driver?)");
-  StemParams p;
+static int plan_stem(const b2_conv_args* a, int BN, ConvPlan* pl) {
+  StemParams& p = pl->p.stem;
   memset(&p, 0, sizeof(p));
   p.T = a->T; p.H = a->H; p.W = a->W;
   p.To = (a->T + 2 * a->pt - a->kt) / a->st + 1;
@@ -568,10 +449,8 @@ static int launch_stem(const b2_conv_args* a, cudaStream_t stream) {
   if (p.ntiles_n * BN > 256) return set_error(B2_ERR_UNSUPPORTED, "stem convolution supports at most 256 output channels");
   p.tiles_w = (p.Wo + kStemTileW - 1) / kStemTileW;
   p.tiles_h = (p.Ho + p.G - 1) / p.G;
-  static int pair_env = -1;
-  if (pair_env < 0) { const char* e = getenv("B2_STEM_PAIR"); pair_env = (e && e[0] == '0') ? 0 : 1; }
   p.planes_total = a->N * p.To;
-  p.pair = (pair_env && a->kt == 1 && a->pt == 0 && p.Wo <= 60 && !a->pool_w && a->W <= 120) ? 1 : 0;
+  p.pair = (tuning().stem_pair && a->kt == 1 && a->pt == 0 && p.Wo <= 60 && !a->pool_w && a->W <= 120) ? 1 : 0;
   const long long plane_items = p.pair ? (p.planes_total + 1) / 2 : p.planes_total;
   const long long items = (long long)p.tiles_w * p.tiles_h * p.ntiles_n * plane_items;
   if (items >= (1ll << 31)) return set_error(B2_ERR_INVALID, "stem problem too large");
@@ -584,31 +463,20 @@ static int launch_stem(const b2_conv_args* a, cudaStream_t stream) {
   p.pool_w = a->pool_w; p.Wp = (p.Wo - 1) / 2 + 1;
   if (a->pool_w && (!a->relu || p.tiles_w != 1))
     return set_error(B2_ERR_UNSUPPORTED, "fused W pooling needs ReLU and an output row of at most %d columns (got %d)", kStemTileW, p.Wo);
-  const int smem_bytes = p.nstages * p.stage_bytes + tail_bytes;
-  B2_OPT_IN_SMEM(stemconv_kernel<BN>, 227 * 1024);
   // input viewed as 8-byte pixels (W, H, N*T); box (256, rows, 1); no swizzle -> dense 2 KB rows in smem
-  CUtensorMap tmX;
-  cuuint64_t dims[3] = {(cuuint64_t)a->W, (cuuint64_t)a->H, (cuuint64_t)a->N * a->T};
-  cuuint64_t strides[2] = {(cuuint64_t)a->W * 8, (cuuint64_t)a->H * a->W * 8};
-  cuuint32_t box[3] = {(cuuint32_t)kStemRowPx, (cuuint32_t)p.rows, 1};
+  TmapSpec& tm = pl->tm[0];
+  tm = TmapSpec{a->x, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, {(cuuint64_t)a->W, (cuuint64_t)a->H, (cuuint64_t)a->N * a->T},
+                {(cuuint64_t)a->W * 8, (cuuint64_t)a->H * a->W * 8}, {(cuuint32_t)kStemRowPx, (cuuint32_t)p.rows, 1}, {1, 1, 1}, false};
   if (p.pair) {      // (W, plane, H): box (128 pixels, 2 planes, rows) -> smem [row][plane][1024 B]
-    dims[1] = (cuuint64_t)a->N * a->T; dims[2] = (cuuint64_t)a->H;
-    strides[0] = (cuuint64_t)a->H * a->W * 8; strides[1] = (cuuint64_t)a->W * 8;
-    box[0] = 128; box[1] = 2; box[2] = (cuuint32_t)p.rows;
+    tm.dims[1] = (cuuint64_t)a->N * a->T; tm.dims[2] = (cuuint64_t)a->H;
+    tm.strides[0] = (cuuint64_t)a->H * a->W * 8; tm.strides[1] = (cuuint64_t)a->W * 8;
+    tm.box[0] = 128; tm.box[1] = 2; tm.box[2] = (cuuint32_t)p.rows;
   }
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(&tmX, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, const_cast<void*>(a->x), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return set_error(B2_ERR_CUDA, "cuTensorMapEncodeTiled(stem) failed (%d)", (int)r);
-  const int grid = p.items_total < sm_count() ? p.items_total : sm_count();
-  B2_CHECK_CUDA(launch_pdl(stemconv_kernel<BN>, dim3(grid), dim3(kStemThreads), smem_bytes, stream, tmX, p));
-  B2_CHECK_LAUNCH("stemconv_kernel");
-  return B2_OK;
+  return set_launch(pl, BN == 64 ? KERN_STEM64 : KERN_STEM128, persistent_grid(p.items_total), kStemThreads, p.nstages * p.stage_bytes + tail_bytes);
 }
 
 // ------------------------------------------------------------------------------------------
-// launcher shared by conv and gemm
+// GEMM-shaped launches shared by convolutions and the GEMM entry points
 // ------------------------------------------------------------------------------------------
 struct IgemmLaunch {
   IgemmParams p;
@@ -622,61 +490,15 @@ struct IgemmLaunch {
   int b_cols;             // logical K extent of B
 };
 
-template <int BN>
-static int launch_igemm(const IgemmLaunch& L, cudaStream_t stream) {
-  using S = IgemmSmem<BN>;
-  B2_OPT_IN_SMEM(igemm_kernel<BN>, S::kTotalBytes);
-  const IgemmParams& p = L.p;
-  CUtensorMap tmA, tmB, tmC, tmR;
-  memset(&tmA, 0, sizeof(tmA)); memset(&tmC, 0, sizeof(tmC)); memset(&tmR, 0, sizeof(tmR));
-  int rc;
-  if ((rc = make_tmap_2d_f16(&tmB, L.w, (uint64_t)L.b_cols, (uint64_t)p.Ncols, (uint64_t)L.ldb, kBK, BN, true)) != B2_OK)
-    return rc;
-  if (p.amode == AMODE_TMA) {
-    if ((rc = make_tmap_2d_f16(&tmA, L.a_mat, (uint64_t)L.a_cols, (uint64_t)p.M_total, (uint64_t)L.lda, kBK, kBM, true)) != B2_OK)
-      return rc;
-  } else {
-    tmA = tmB;
-  }
-  if (p.epi == EPI_TMA_F16) {
-    if ((rc = make_tmap_2d_f16(&tmC, p.y, (uint64_t)p.ldy, (uint64_t)p.M_total, (uint64_t)p.ldy, 64, kBM, true)) != B2_OK)
-      return rc;
-    if (p.residual) {
-      if ((rc = make_tmap_2d_f16(&tmR, p.residual, (uint64_t)p.ldr, (uint64_t)p.M_total, (uint64_t)p.ldr, 64, kBM, true)) != B2_OK)
-        return rc;
-    } else {
-      tmR = tmC;
-    }
-  } else {
-    tmC = tmB; tmR = tmB;
-  }
-  dim3 grid((p.epi == EPI_TMA_F16 ? (p.ldy + BN - 1) / BN : (p.Ncols + BN - 1) / BN), (p.M_total + kBM - 1) / kBM, 1);
-  B2_CHECK_CUDA(launch_pdl(igemm_kernel<BN>, grid, dim3(kThreads), S::kTotalBytes, stream, tmA, tmB, tmC, tmR, p));
-  B2_CHECK_LAUNCH("igemm_kernel");
-  return B2_OK;
-}
-
-
-// ------------------------------------------------------------------------------------------
-// small-M path: dense-M implicit GEMM, split-K over a thread-block cluster (b2_densem.cuh)
-// ------------------------------------------------------------------------------------------
 // Which layers take the dense-M kernel (measured with tools/conv_sweep.py as CUDA-graph replays, profiles/smallm_sweep_r02.txt):
 // it beats the slab kernel only where a plane fills a small part of a 128-row tile AND the K loop is long enough to split --
 // stride-1 multi-tap convolutions with M <= 1024 output positions (4x4 planes: 12% tile fill), strided multi-tap convolutions
 // (whose slab form needs four phase sub-images per tap) with M <= 8192.  1x1x1 convolutions stay on the persistent GEMM.
-// B2_DENSEM_MAXM = 0 disables the path, a positive value replaces BOTH thresholds (debug / sweeps).
-static int g_densem_maxm = -1;
-static int densem_maxm_env() {
-  if (g_densem_maxm < 0) {
-    const char* e = getenv("B2_DENSEM_MAXM");
-    g_densem_maxm = e ? atoi(e) : -2;               // -2: no override
-    if (g_densem_maxm == -1) g_densem_maxm = -2;
-  }
-  return g_densem_maxm;
-}
+// Only plain per-column affines without the generator's extras qualify; the callers test that.
 static bool densem_wanted(long long M, int taps, bool strided) {
-  const int ov = densem_maxm_env();
-  if (ov >= 0) return ov > 0 && M <= ov;
+  const Tuning& t = tuning();
+  if (t.gemm_algo != 0) return false;
+  if (t.densem_maxm >= 0) return t.densem_maxm > 0 && M <= t.densem_maxm;
   if (taps <= 1) return false;
   return strided ? M <= 8192 : M <= 1024;
 }
@@ -688,109 +510,67 @@ static bool densem_split_ok(int bn, int S, int nkb) {      // bn / S a multiple 
   const int per = (nkb + S - 1) / S;
   return (S - 1) * per < nkb;
 }
-static int g_densem_force_s = -1;
-static void densem_plan(int M, int ldy, int nkb, int* bn_out, int* S_out) {
-  int best_bn = 256, best_waste = 1 << 30;
-  for (int bn = 256; bn >= 64; bn -= 32) {
-    const int tn = (ldy + bn - 1) / bn;
-    const int waste = tn * bn - ldy;
-    if (waste < best_waste) { best_waste = waste; best_bn = bn; }
+static int plan_densem(const IgemmLaunch& L, ConvPlan* pl) {
+  const IgemmParams& p = L.p;
+  const int width = (p.epi == EPI_DIRECT_F32) ? p.Ncols : p.ldy;
+  int bn = 256, best_waste = 1 << 30;
+  for (int c = 256; c >= 64; c -= 32) {
+    const int waste = (width + c - 1) / c * c - width;
+    if (waste < best_waste) { best_waste = waste; bn = c; }
   }
-  if (ldy <= 32) best_bn = 32;
-  const int tiles = ((M + 127) / 128) * ((ldy + best_bn - 1) / best_bn);
-  if (g_densem_force_s < 0) { const char* e = getenv("B2_DENSEM_S"); g_densem_force_s = e ? atoi(e) : 0; }
+  if (width <= 32) bn = 32;
+  const int tiles = ((p.M_total + 127) / 128) * ((width + bn - 1) / bn);
+  const int force_s = tuning().densem_s;
   int S = 1;
   for (int cand = 1; cand <= 8; ++cand) {
-    if (!densem_split_ok(best_bn, cand, nkb) || (cand > 1 && nkb / cand < 2)) continue;
-    if (g_densem_force_s > 0) { if (cand <= g_densem_force_s) S = cand; continue; }
+    if (!densem_split_ok(bn, cand, p.nkb) || (cand > 1 && p.nkb / cand < 2)) continue;
+    if (force_s > 0) { if (cand <= force_s) S = cand; continue; }
     S = cand;
     if (tiles * cand >= 64) break;                  // measured: beyond ~half the SMs the cluster / DSMEM cost outgrows the gain
   }
-  *bn_out = best_bn; *S_out = S;
-}
-
-static int launch_densem(const IgemmLaunch& L, cudaStream_t stream) {
-  DensemParams dp;
+  DensemParams& dp = pl->p.densem;
   memset(&dp, 0, sizeof(dp));
-  dp.g = L.p;
-  const IgemmParams& p = L.p;
-  const int width = (p.epi == EPI_DIRECT_F32) ? p.Ncols : p.ldy;
-  int bn = 0, S = 1;
-  densem_plan(p.M_total, width, p.nkb, &bn, &S);
+  dp.g = p;
   dp.bn = bn; dp.bbytes = bn * 128; dp.stage_bytes = kBM * kBK * 2 + dp.bbytes;
   dp.tmem_cols = bn <= 32 ? 32 : bn <= 64 ? 64 : bn <= 128 ? 128 : 256;
   dp.ksplit = S;
   dp.kb_per = (p.nkb + S - 1) / S;
   dp.nstages = (227 * 1024 - 256 - 1024) / dp.stage_bytes;
   if (dp.nstages > kDmMaxStages) dp.nstages = kDmMaxStages;
-  const int smem_bytes = dp.nstages * dp.stage_bytes + 256 + 1024;
-  B2_OPT_IN_SMEM(densem_kernel, 227 * 1024);
-  CUtensorMap tmA, tmB;
-  int rc;
-  if ((rc = make_tmap_2d_f16(&tmB, L.w, (uint64_t)L.b_cols, (uint64_t)p.Ncols, (uint64_t)L.ldb, kBK, (uint32_t)bn, true)) != B2_OK) return rc;
-  if (p.amode == AMODE_TMA) {
-    if ((rc = make_tmap_2d_f16(&tmA, L.a_mat, (uint64_t)L.a_cols, (uint64_t)p.M_total, (uint64_t)L.lda, kBK, kBM, true)) != B2_OK) return rc;
-  } else {
-    tmA = tmB;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((width + bn - 1) / bn, (p.M_total + kBM - 1) / kBM, dp.ksplit);
-  cfg.blockDim = dim3(kDmThreads);
-  cfg.dynamicSmemBytes = smem_bytes;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-  attr[1].id = cudaLaunchAttributeClusterDimension;
-  attr[1].val.clusterDim.x = 1; attr[1].val.clusterDim.y = 1; attr[1].val.clusterDim.z = dp.ksplit;
-  cfg.attrs = attr; cfg.numAttrs = 2;
-  B2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, densem_kernel, tmA, tmB, dp));
-  B2_CHECK_LAUNCH("densem_kernel");
-  return B2_OK;
+  B2_TRY(tmap_2d_f16(&pl->tm[1], L.w, (uint64_t)L.b_cols, (uint64_t)p.Ncols, (uint64_t)L.ldb, kBK, (uint32_t)bn, true));
+  if (p.amode == AMODE_TMA) B2_TRY(tmap_2d_f16(&pl->tm[0], L.a_mat, (uint64_t)L.a_cols, (uint64_t)p.M_total, (uint64_t)L.lda, kBK, kBM, true));
+  else pl->tm_copy[0] = 1;
+  return set_launch(pl, KERN_DENSEM, dim3((width + bn - 1) / bn, (p.M_total + kBM - 1) / kBM, S), kDmThreads,
+                    dp.nstages * dp.stage_bytes + 256 + 1024, S);
 }
 
-// does the dense-M kernel take this launch?  (plain per-column affine, no generator extras, few output positions)
-static bool densem_applies(const IgemmParams& p, int k2) {
-  if (p.in_scale) return false;
-  const bool gather = p.amode != AMODE_TMA;
-  const int taps = gather ? p.kt * p.kh * p.kw : 1;
-  const bool strided = gather && (p.st > 1 || p.sh > 1 || p.sw > 1);
-  return k2 == 0 && !p.aff_ld && !p.res_up && !p.res_pre && !p.y2 && densem_wanted(p.M_total, taps, strided) &&
-         (p.epi == EPI_DIRECT_F32 || !p.per_row);
-}
-
-static int g_gemm_algo = 0;   // 0 auto (persistent kernel where it applies), 1 force the per-tile kernel
-
-template <int BN, int GAN>
-static int launch_pgemm(const IgemmLaunch& L, cudaStream_t stream) {
-  using S = PgemmSmem<BN>;
-  B2_OPT_IN_SMEM((pgemm_kernel<BN, GAN>), S::kTotal);
+static int plan_pgemm(const IgemmLaunch& L, int BN, bool gan, ConvPlan* pl) {
   const IgemmParams& ip = L.p;
-  CUtensorMap tmA, tmB, tmC, tmR;
-  int rc;
-  if ((rc = make_tmap_2d_f16(&tmA, L.a_mat, (uint64_t)L.a_cols, (uint64_t)ip.M_total, (uint64_t)L.lda, 64, 128, true)) != B2_OK) return rc;
-  if ((rc = make_tmap_2d_f16(&tmB, L.w, (uint64_t)L.b_cols, (uint64_t)ip.Ncols, (uint64_t)L.ldb, 64, BN, true)) != B2_OK) return rc;
-  if ((rc = make_tmap_2d_f16(&tmC, ip.y, (uint64_t)ip.ldy, (uint64_t)ip.M_total, (uint64_t)ip.ldy, 64, 128, true)) != B2_OK) return rc;
+  B2_TRY(tmap_2d_f16(&pl->tm[0], L.a_mat, (uint64_t)L.a_cols, (uint64_t)ip.M_total, (uint64_t)L.lda, 64, 128, true));
+  B2_TRY(tmap_2d_f16(&pl->tm[1], L.w, (uint64_t)L.b_cols, (uint64_t)ip.Ncols, (uint64_t)L.ldb, 64, BN, true));
+  B2_TRY(tmap_2d_f16(&pl->tm[4], ip.y, (uint64_t)ip.ldy, (uint64_t)ip.M_total, (uint64_t)ip.ldy, 64, 128, true));
   const int up_W = ip.up_W > 0 ? ip.up_W : 2;
   const int res_rows = up_W >= 128 ? 64 : 32;
   if (ip.residual && ip.res_up) {
     // low-res skip tensor: a tile's 128 output rows read res_rows consecutive rows of it (see PgemmParams::res_up)
     if (!(up_W % 128 == 0 || (up_W <= 64 && 64 % up_W == 0)))
       return set_error(B2_ERR_UNSUPPORTED, "residual_up needs an output width that is a multiple of 128 or divides 64 (got %d)", up_W);
-    if ((rc = make_tmap_2d_f16(&tmR, ip.residual, (uint64_t)ip.ldr, (uint64_t)ip.M_total / 4, (uint64_t)ip.ldr, 64, res_rows, true)) != B2_OK) return rc;
+    B2_TRY(tmap_2d_f16(&pl->tm[5], ip.residual, (uint64_t)ip.ldr, (uint64_t)ip.M_total / 4, (uint64_t)ip.ldr, 64, res_rows, true));
   } else if (ip.residual) {
-    if ((rc = make_tmap_2d_f16(&tmR, ip.residual, (uint64_t)ip.ldr, (uint64_t)ip.M_total, (uint64_t)ip.ldr, 64, 128, true)) != B2_OK) return rc;
+    B2_TRY(tmap_2d_f16(&pl->tm[5], ip.residual, (uint64_t)ip.ldr, (uint64_t)ip.M_total, (uint64_t)ip.ldr, 64, 128, true));
   } else {
-    tmR = tmC;
+    pl->tm_copy[5] = 4;
   }
-  CUtensorMap tmC2 = tmC;
-  if (ip.y2 && (rc = make_tmap_2d_f16(&tmC2, ip.y2, (uint64_t)ip.ldy, (uint64_t)ip.M_total, (uint64_t)ip.ldy, 64, 128, true)) != B2_OK) return rc;
-  CUtensorMap tmA2 = tmA, tmB2 = tmB;
+  if (ip.y2) B2_TRY(tmap_2d_f16(&pl->tm[6], ip.y2, (uint64_t)ip.ldy, (uint64_t)ip.M_total, (uint64_t)ip.ldy, 64, 128, true));
+  else pl->tm_copy[6] = 4;
   if (L.k2 > 0) {
-    if ((rc = make_tmap_2d_f16(&tmA2, L.a2, (uint64_t)L.k2, (uint64_t)ip.M_total, (uint64_t)L.lda2, 64, 128, true)) != B2_OK) return rc;
-    if ((rc = make_tmap_2d_f16(&tmB2, L.w2, (uint64_t)L.k2, (uint64_t)ip.Ncols, (uint64_t)L.ldb2, 64, BN, true)) != B2_OK) return rc;
+    B2_TRY(tmap_2d_f16(&pl->tm[2], L.a2, (uint64_t)L.k2, (uint64_t)ip.M_total, (uint64_t)L.lda2, 64, 128, true));
+    B2_TRY(tmap_2d_f16(&pl->tm[3], L.w2, (uint64_t)L.k2, (uint64_t)ip.Ncols, (uint64_t)L.ldb2, 64, BN, true));
+  } else {
+    pl->tm_copy[2] = 0; pl->tm_copy[3] = 1;
   }
-  PgemmParams p;
+  PgemmParams& p = pl->p.pgemm;
+  p = PgemmParams{};
   p.M = ip.M_total; p.Ncols = ip.Ncols; p.ldy = ip.ldy; p.nkb = ip.nkb;
   p.nkb2 = (L.k2 + 63) / 64;
   p.tiles_n = (ip.ldy + BN - 1) / BN;
@@ -803,99 +583,245 @@ static int launch_pgemm(const IgemmLaunch& L, cudaStream_t stream) {
   p.res_ld = ip.ldr; p.Wh = up_W; p.Hh = ip.up_H > 0 ? ip.up_H : 2; p.res_rows = res_rows;
   p.fd_Wh = make_fastdiv(p.Wh); p.fd_Hh = make_fastdiv(p.Hh);
   p.res_pre = ip.res_pre;
-  p.in_scale = GAN ? ip.in_scale : nullptr; p.in_shift = ip.in_shift; p.in_ld = ip.in_ld; p.in_rows = ip.in_rows > 0 ? ip.in_rows : 128;
+  p.in_scale = gan ? ip.in_scale : nullptr; p.in_shift = ip.in_shift; p.in_ld = ip.in_ld; p.in_rows = ip.in_rows > 0 ? ip.in_rows : 128;
   p.dual = ip.y2 != nullptr; p.scale2 = ip.scale2; p.shift2 = ip.shift2; p.aff2_ld = ip.aff2_ld; p.aff2_rows = ip.aff2_rows > 0 ? ip.aff2_rows : 128;
-  const int grid = p.tiles_total < sm_count() ? p.tiles_total : sm_count();
-  B2_CHECK_CUDA(launch_pdl(pgemm_kernel<BN, GAN>, dim3(grid), dim3(GAN ? kPgThreadsGan : kPgThreads), S::kTotal, stream, tmA, tmB, tmA2, tmB2, tmC, tmR, tmC2, p));
-  B2_CHECK_LAUNCH("pgemm_kernel");
+  const int kernel = BN == 64 ? (gan ? KERN_PGEMM64_GAN : KERN_PGEMM64) : (gan ? KERN_PGEMM128_GAN : KERN_PGEMM128);
+  return set_launch(pl, kernel, persistent_grid(p.tiles_total), gan ? kPgThreadsGan : kPgThreads,
+                    BN == 64 ? PgemmSmem<64>::kTotal : PgemmSmem<128>::kTotal);
+}
+
+static int plan_igemm(const IgemmLaunch& L, ConvPlan* pl) {
+  const IgemmParams& p = L.p;
+  // 64-wide tiles for narrow outputs, 128 otherwise
+  const int BN = ((p.epi == EPI_TMA_F16) ? p.ldy : p.Ncols) <= 64 ? 64 : 128;
+  B2_TRY(tmap_2d_f16(&pl->tm[1], L.w, (uint64_t)L.b_cols, (uint64_t)p.Ncols, (uint64_t)L.ldb, kBK, BN, true));
+  if (p.amode == AMODE_TMA) B2_TRY(tmap_2d_f16(&pl->tm[0], L.a_mat, (uint64_t)L.a_cols, (uint64_t)p.M_total, (uint64_t)L.lda, kBK, kBM, true));
+  else pl->tm_copy[0] = 1;
+  if (p.epi == EPI_TMA_F16) {
+    B2_TRY(tmap_2d_f16(&pl->tm[2], p.y, (uint64_t)p.ldy, (uint64_t)p.M_total, (uint64_t)p.ldy, 64, kBM, true));
+    if (p.residual) B2_TRY(tmap_2d_f16(&pl->tm[3], p.residual, (uint64_t)p.ldr, (uint64_t)p.M_total, (uint64_t)p.ldr, 64, kBM, true));
+    else pl->tm_copy[3] = 2;
+  } else {
+    pl->tm_copy[2] = 1; pl->tm_copy[3] = 1;
+  }
+  pl->p.igemm = p;
+  return set_launch(pl, BN == 64 ? KERN_IGEMM64 : KERN_IGEMM128,
+                    dim3((p.epi == EPI_TMA_F16 ? (p.ldy + BN - 1) / BN : (p.Ncols + BN - 1) / BN), (p.M_total + kBM - 1) / kBM, 1),
+                    kThreads, BN == 64 ? IgemmSmem<64>::kTotalBytes : IgemmSmem<128>::kTotalBytes);
+}
+
+// dense_m: the caller found the launch plain and small enough for the dense-M kernel
+static int plan_gemm_shaped(const IgemmLaunch& L, bool dense_m, ConvPlan* pl) {
+  const IgemmParams& p = L.p;
+  if (dense_m) return plan_densem(L, pl);
+  if (tuning().gemm_algo == 0 && p.amode == AMODE_TMA && p.epi == EPI_TMA_F16 && !p.per_row) {
+    // the generator's extras need the GAN instance; a second output needs the 64-wide one (it has a second staging tile)
+    const bool gan = p.y2 || p.res_up || p.res_pre || p.in_scale;
+    return plan_pgemm(L, (p.y2 || p.ldy <= 64) ? 64 : 128, gan, pl);
+  }
+  if (p.aff_ld)
+    return set_error(B2_ERR_UNSUPPORTED, "per-sample affine is implemented by the slab convolution and the persistent GEMM only");
+  if (p.res_up || p.res_pre || p.y2 || p.in_scale)
+    return set_error(B2_ERR_UNSUPPORTED, "upsampled / pre-scale residuals, second outputs and input affines are implemented by the persistent GEMM (1x1 convolutions, fp16) only");
+  return plan_igemm(L, pl);
+}
+
+// ------------------------------------------------------------------------------------------
+// the planners of the entry points, and the launcher
+// ------------------------------------------------------------------------------------------
+static int conv_out_dim(int in, int k, int s, int p) { return (in + 2 * p - k) / s + 1; }
+
+// Order: dense-M pre-check -> temporal stack -> temporal-group slab -> slab -> stem / 1x1x1 / gather GEMM.
+static int plan_conv(const b2_conv_args* a, ConvPlan* pl) {
+  pl->kernel = KERN_NONE;
+  memset(pl->tm_copy, -1, sizeof(pl->tm_copy));
+  const Tuning& t = tuning();
+  const int To = conv_out_dim(a->T, a->kt, a->st, a->pt), Ho = conv_out_dim(a->H, a->kh, a->sh, a->ph),
+            Wo = conv_out_dim(a->W, a->kw, a->sw, a->pw);
+  const int taps = a->kt * a->kh * a->kw;
+  const bool extras = a->aff_ld || a->y2 || a->residual_up || a->residual_pre || a->in_scale;
+  // a plain convolution: what the temporal stack / temporal-group kernels (and the dense-M kernel, fp32 output aside) implement
+  const bool plain = a->mode == B2_CONV_AUTO && !a->out_f32 && !a->upsample && !extras;
+  const bool dense_m = a->mode == B2_CONV_AUTO && !a->upsample && !extras &&
+                       densem_wanted((long long)a->N * To * Ho * Wo, taps, a->st > 1 || a->sh > 1 || a->sw > 1);
+  int rc;
+  if (!dense_m && t.conv_algo == 0) {
+    if (plain && ((rc = plan_tstack(a, pl)) != B2_OK || pl->kernel != KERN_NONE)) return rc;
+    if (plain && ((rc = plan_slabts(a, pl)) != B2_OK || pl->kernel != KERN_NONE)) return rc;
+    if ((rc = plan_slab(a, pl)) != B2_OK || pl->kernel != KERN_NONE) return rc;
+  }
+  if (a->upsample) return set_error(B2_ERR_UNSUPPORTED, "fused upsampling needs the slab kernel, which does not take this shape");
+
+  IgemmLaunch L;
+  memset(&L, 0, sizeof(L));
+  IgemmParams& p = L.p;
+  p.x = reinterpret_cast<const __half*>(a->x);
+  p.N = a->N; p.T = a->T; p.H = a->H; p.W = a->W; p.C = a->C;
+  p.To = To; p.Ho = Ho; p.Wo = Wo;
+  p.kt = a->kt; p.kh = a->kh; p.kw = a->kw;
+  p.st = a->st; p.sh = a->sh; p.sw = a->sw;
+  p.pt = a->pt; p.ph = a->ph; p.pw = a->pw;
+  const long long M = (long long)a->N * p.To * p.Ho * p.Wo;
+  B2_CHECK_ARG(M < (1ll << 31), "output too large");
+  p.M_total = (int)M;
+  p.Ncols = a->K;
+  p.scale = a->scale; p.shift = a->shift;
+  p.residual = reinterpret_cast<const __half*>(a->residual);
+  p.ldr = a->ldr;
+  p.y = a->y; p.ldy = a->ldy;
+  p.relu = a->relu; p.per_row = 0; p.accumulate = a->accumulate;
+  p.epi = a->out_f32 ? EPI_DIRECT_F32 : EPI_TMA_F16;
+  p.aff_ld = a->aff_ld;
+  p.res_up = a->residual_up; p.res_pre = a->residual_pre; p.up_H = p.Ho; p.up_W = p.Wo;
+  p.y2 = a->y2; p.scale2 = a->scale2; p.shift2 = a->shift2; p.aff2_ld = a->aff2_ld; p.aff2_rows = p.To * p.Ho * p.Wo;
+  if (a->y2) {
+    B2_CHECK_ARG(a->scale2 && a->shift2 && a->aff2_ld >= a->K && !a->out_f32 && taps == 1,
+                 "second output needs scale2 / shift2 (fp32 [N][aff2_ld >= K]) and a 1x1 convolution with fp16 output");
+    if (p.aff2_rows % 128 != 0)
+      return set_error(B2_ERR_UNSUPPORTED, "second output with a per-sample affine needs To*Ho*Wo %% 128 == 0 (got %d)", p.aff2_rows);
+  }
+  if (a->in_scale) {
+    B2_CHECK_ARG(a->in_shift && a->in_aff_ld >= a->C && (a->in_aff_ld & 3) == 0 && !a->out_f32 && taps == 1 && a->st == 1 &&
+                     a->sh == 1 && a->sw == 1 && (reinterpret_cast<uintptr_t>(a->in_scale) & 15) == 0 &&
+                     (reinterpret_cast<uintptr_t>(a->in_shift) & 15) == 0,
+                 "input affine needs in_shift, a 16-byte aligned fp32 [N][in_aff_ld >= C] pair (pitch %% 4 == 0) and a 1x1 stride-1 convolution with fp16 output");
+    if ((p.To * p.Ho * p.Wo) % 128 != 0 || a->C % 64 != 0)
+      return set_error(B2_ERR_UNSUPPORTED, "input affine needs To*Ho*Wo %% 128 == 0 and a channel pitch that is a multiple of 64 (got %d, %d)",
+                       p.To * p.Ho * p.Wo, a->C);
+    p.in_scale = a->in_scale; p.in_shift = a->in_shift; p.in_ld = a->in_aff_ld; p.in_rows = p.To * p.Ho * p.Wo;
+  }
+  p.aff_rows = p.To * p.Ho * p.Wo;
+  if (a->aff_ld && p.aff_rows % 128 != 0)
+    return set_error(B2_ERR_UNSUPPORTED, "per-sample affine on a 1x1x1 convolution needs To*Ho*Wo %% 128 == 0 (got %d)", p.aff_rows);
+  L.w = a->w;
+
+  if (a->mode == B2_CONV_STEM7) {
+    B2_CHECK_ARG(!a->out_f32 && a->residual == nullptr, "stem convolution has no residual / fp32 output");
+    B2_CHECK_ARG(a->st == 1 && a->sh == 2, "stem convolution needs strides (1, 2, 2)");
+    return plan_stem(a, a->K <= 64 ? 64 : 128, pl);
+  } else if (taps == 1 && a->st == 1 && a->sh == 1 && a->sw == 1 && a->pt == 0 && a->ph == 0 && a->pw == 0) {
+    // 1x1x1 stride-1: A is literally the [M][C] activation matrix -> TMA on both operands
+    p.amode = AMODE_TMA;
+    p.nkb = (a->C + kBK - 1) / kBK;
+    L.a_mat = a->x; L.lda = a->C; L.a_cols = a->C;
+    L.ldb = a->C; L.b_cols = a->C;
+  } else {
+    p.amode = AMODE_GATHER;
+    p.cchunks = (a->C + kBK - 1) / kBK;
+    p.nkb = taps * p.cchunks;
+    L.ldb = taps * a->C;
+    L.b_cols = L.ldb;
+    // When C % 64 != 0 the last K block of a tap also covers the first columns of the next tap's
+    // weights; the activation side zero-fills channels >= C, so those products vanish.
+  }
+  return plan_gemm_shaped(L, dense_m, pl);
+}
+
+static int plan_gemm(const b2_gemm_args* g, const void* a2, int lda2, const void* b2, int ldb2, int k2, ConvPlan* pl) {
+  pl->kernel = KERN_NONE;
+  memset(pl->tm_copy, -1, sizeof(pl->tm_copy));
+  IgemmLaunch L;
+  memset(&L, 0, sizeof(L));
+  IgemmParams& p = L.p;
+  p.amode = AMODE_TMA;
+  p.M_total = g->M;
+  p.Ncols = g->N;
+  p.nkb = (g->Kd + kBK - 1) / kBK;
+  p.scale = g->scale; p.shift = g->shift;
+  p.residual = reinterpret_cast<const __half*>(g->residual);
+  p.ldr = g->ldr;
+  p.y = g->d; p.ldy = g->ldd;
+  p.relu = g->relu; p.per_row = g->per_row; p.accumulate = g->accumulate;
+  p.epi = g->out_f32 ? EPI_DIRECT_F32 : EPI_TMA_F16;
+  B2_CHECK_ARG(g->aff_ld >= 0 && (g->aff_ld == 0 || (g->aff_ld >= g->N && g->aff_rows > 0 && g->aff_rows % 128 == 0 &&
+                                                     !g->out_f32 && !g->per_row)),
+               "bad per-sample affine (pitch %d, rows per sample %d)", g->aff_ld, g->aff_rows);
+  p.aff_ld = g->aff_ld; p.aff_rows = g->aff_rows;
+  if (g->d2) {
+    B2_CHECK_ARG(g->scale2 && g->shift2 && g->aff2_ld >= g->N && g->aff2_rows > 0 && g->aff2_rows % 128 == 0 && !g->out_f32 && !g->per_row,
+                 "second output needs scale2 / shift2 (fp32 [M / aff2_rows][aff2_ld >= N], aff2_rows %% 128 == 0) and fp16 output");
+    p.y2 = g->d2; p.scale2 = g->scale2; p.shift2 = g->shift2; p.aff2_ld = g->aff2_ld; p.aff2_rows = g->aff2_rows;
+  }
+  p.x = reinterpret_cast<const __half*>(g->a);
+  L.a_mat = g->a; L.lda = g->lda; L.a_cols = g->Kd;
+  L.w = g->b; L.ldb = g->ldb; L.b_cols = g->Kd;
+  L.a2 = a2; L.lda2 = lda2; L.w2 = b2; L.ldb2 = ldb2; L.k2 = k2;
+  if (k2 > 0 && tuning().gemm_algo != 0) return set_error(B2_ERR_UNSUPPORTED, "two-operand GEMM needs the persistent kernel");
+  const bool dense_m = k2 == 0 && !g->aff_ld && !g->d2 && (g->out_f32 || !g->per_row) && densem_wanted(g->M, 1, false);
+  return plan_gemm_shaped(L, dense_m, pl);
+}
+
+static int launch_plan(const ConvPlan& pl, cudaStream_t stream) {
+  CUtensorMap tm[kMaxTmaps];
+  for (int i = 0; i < kNumTmaps[pl.kernel]; ++i)
+    if (pl.tm_copy[i] < 0) B2_TRY(encode_tmap(&tm[i], pl.tm[i]));
+  for (int i = 0; i < kNumTmaps[pl.kernel]; ++i)
+    if (pl.tm_copy[i] >= 0) tm[i] = tm[pl.tm_copy[i]];
+  const dim3 g = pl.grid, b = pl.block;
+  const size_t smem = (size_t)pl.smem;
+  cudaError_t e = cudaSuccess;
+  // shared memory opt-in (once per kernel and device), then the launch with programmatic stream serialization
+#define B2_RUN(kernel, optin, ...) B2_OPT_IN_SMEM(kernel, optin); e = launch_pdl(kernel, g, b, smem, stream, __VA_ARGS__); break
+  switch (pl.kernel) {
+    case KERN_TSTACK: B2_RUN(tstack_kernel, 227 * 1024, tm[0], tm[1], pl.p.tstack);
+    case KERN_SLABTS: B2_RUN(slabts_kernel, 227 * 1024, tm[0], tm[1], pl.p.slab);
+    case KERN_SLAB64: B2_RUN(slabconv_kernel<64>, 227 * 1024, tm[0], tm[1], pl.p.slab);
+    case KERN_SLAB128: B2_RUN(slabconv_kernel<128>, 227 * 1024, tm[0], tm[1], pl.p.slab);
+    case KERN_SLABN: B2_RUN(slabconv_kernel<0>, 227 * 1024, tm[0], tm[1], pl.p.slab);
+    case KERN_STEM64: B2_RUN(stemconv_kernel<64>, 227 * 1024, tm[0], pl.p.stem);
+    case KERN_STEM128: B2_RUN(stemconv_kernel<128>, 227 * 1024, tm[0], pl.p.stem);
+    case KERN_PGEMM64: B2_RUN((pgemm_kernel<64, 0>), PgemmSmem<64>::kTotal, tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], tm[6], pl.p.pgemm);
+    case KERN_PGEMM64_GAN: B2_RUN((pgemm_kernel<64, 1>), PgemmSmem<64>::kTotal, tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], tm[6], pl.p.pgemm);
+    case KERN_PGEMM128: B2_RUN((pgemm_kernel<128, 0>), PgemmSmem<128>::kTotal, tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], tm[6], pl.p.pgemm);
+    case KERN_PGEMM128_GAN: B2_RUN((pgemm_kernel<128, 1>), PgemmSmem<128>::kTotal, tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], tm[6], pl.p.pgemm);
+    case KERN_IGEMM64: B2_RUN(igemm_kernel<64>, IgemmSmem<64>::kTotalBytes, tm[0], tm[1], tm[2], tm[3], pl.p.igemm);
+    case KERN_IGEMM128: B2_RUN(igemm_kernel<128>, IgemmSmem<128>::kTotalBytes, tm[0], tm[1], tm[2], tm[3], pl.p.igemm);
+    case KERN_DENSEM: {     // split-K over a thread-block cluster along z
+      B2_OPT_IN_SMEM(densem_kernel, 227 * 1024);
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = g; cfg.blockDim = b; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+      cudaLaunchAttribute attr[2];
+      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+      attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+      attr[1].id = cudaLaunchAttributeClusterDimension;
+      attr[1].val.clusterDim.x = 1; attr[1].val.clusterDim.y = 1; attr[1].val.clusterDim.z = pl.cluster;
+      cfg.attrs = attr; cfg.numAttrs = 2;
+      e = cudaLaunchKernelEx(&cfg, densem_kernel, tm[0], tm[1], pl.p.densem);
+      break;
+    }
+    default: return set_error(B2_ERR_INVALID, "no kernel planned");
+  }
+#undef B2_RUN
+  if (e != cudaSuccess) return set_error(B2_ERR_CUDA, "launch of %s failed: %s", kKernelName[pl.kernel], cudaGetErrorString(e));
+  B2_CHECK_LAUNCH(kKernelName[pl.kernel]);
   return B2_OK;
 }
 
-static int dispatch_igemm(const IgemmLaunch& L, cudaStream_t stream) {
-  if (g_gemm_algo == 0 && densem_applies(L.p, L.k2)) return launch_densem(L, stream);
-  if (g_gemm_algo == 0 && L.p.amode == AMODE_TMA && L.p.epi == EPI_TMA_F16 && !L.p.per_row) {
-    if (L.p.y2) return launch_pgemm<64, 1>(L, stream);       // second output: the 64-wide instance has a second staging tile
-    if (L.p.res_up || L.p.res_pre || L.p.in_scale)
-      return L.p.ldy <= 64 ? launch_pgemm<64, 1>(L, stream) : launch_pgemm<128, 1>(L, stream);
-    return L.p.ldy <= 64 ? launch_pgemm<64, 0>(L, stream) : launch_pgemm<128, 0>(L, stream);
+// Host-only view of a plan for the b2_debug_*_plan entry points; fields the kernel does not have stay 0:
+// {kernel, grid x, y, z, block, smem, cluster, bn, MT, R, PW, WC, wchunks, items, flex, remap, groups, tiles, cchunks, wbytes, S}
+constexpr int kPlanFields = 21;
+static int plan_view(const ConvPlan& pl, int kt_in, int* out, int n) {
+  int v[kPlanFields] = {pl.kernel, (int)pl.grid.x, (int)pl.grid.y, (int)pl.grid.z, (int)pl.block.x, pl.smem, pl.cluster};
+  if (pl.kernel >= KERN_SLABTS && pl.kernel <= KERN_SLABN) {
+    const SlabParams& s = pl.p.slab;
+    const int slab[] = {s.bn, s.MT, s.R, s.PW, s.WC, s.wchunks, s.items_total, pl.kernel == KERN_SLABN, s.kt != kt_in};
+    memcpy(v + 7, slab, sizeof(slab));
+    v[18] = s.cchunks;
+  } else if (pl.kernel == KERN_TSTACK) {
+    const TstackParams& s = pl.p.tstack;
+    v[13] = s.items_total; v[16] = s.groups; v[17] = s.tiles_q; v[18] = s.cchunks; v[19] = s.cchunks * s.kt * kTkWBlock;
+  } else if (pl.kernel == KERN_DENSEM) {
+    v[7] = pl.p.densem.bn; v[20] = pl.p.densem.ksplit;
   }
-  if (L.p.aff_ld)
-    return set_error(B2_ERR_UNSUPPORTED, "per-sample affine is implemented by the slab convolution and the persistent GEMM only");
-  if (L.p.res_up || L.p.res_pre || L.p.y2 || L.p.in_scale)
-    return set_error(B2_ERR_UNSUPPORTED, "upsampled / pre-scale residuals, second outputs and input affines are implemented by the persistent GEMM (1x1 convolutions, fp16) only");
-  // 64-wide tiles for narrow outputs, 128 otherwise
-  const int width = (L.p.epi == EPI_TMA_F16) ? L.p.ldy : L.p.Ncols;
-  if (width <= 64) return launch_igemm<64>(L, stream);
-  return launch_igemm<128>(L, stream);
+  for (int i = 0; i < n; ++i) out[i] = i < kPlanFields ? v[i] : 0;
+  return B2_OK;
 }
 
-bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("B2_PDL"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
-}
+static int g_last_conv_kernel = KERN_NONE;   // kernel of the last b2_conv_ndhwc_fprop launch (tests pin the dispatch)
 
 }  // namespace b2
 
 using namespace b2;
-
-extern "C" {
-
-int b2_version(void) { return 103; }   // 103: split-K / fused (2+1)D / pooled-stem entry points (round 2); 102: generator fields
-/* debug knob (not in the public header): 0 = auto, 1 = never use the slab kernel */
-int b2_debug_set_conv_algo(int algo) { g_conv_algo = algo; return B2_OK; }
-int b2_debug_set_gemm_algo(int algo) { g_gemm_algo = algo; return B2_OK; }
-/* host-only view of the slab kernel's tiling decision for a convolution (no launch, no GPU needed): out = {applies, BN, MT, R, PW,
-   WC, wchunks, items, flex, remapped}.  Used by tests/test_host_logic.py and by tuning scripts. */
-int b2_debug_slab_plan(const b2_conv_args* a_in, int* out) {
-  b2_conv_args remap = *a_in;
-  const b2_conv_args* a = a_in;
-  int wc_hint = 0, remapped = 0;
-  if (a_in->kt > 1 && a_in->kh == 1 && a_in->kw == 1 && a_in->st == 1 && a_in->sh == 1 && a_in->sw == 1 && a_in->ph == 0 && a_in->pw == 0) {
-    remap.T = 1; remap.H = a_in->T; remap.W = a_in->H * a_in->W; remap.kt = 1; remap.kh = a_in->kt; remap.kw = 1;
-    remap.pt = 0; remap.ph = a_in->pt; remap.pw = 0; a = &remap; wc_hint = 64; remapped = 1;
-  }
-  const int wc_try[3] = {wc_hint, 128, 64};
-  int BN = 0, best_mt = 0, best_R = 0; bool flex = false; double best_cost = 0.0; SlabParams best_p;
-  memset(&best_p, 0, sizeof(best_p));
-  for (int attempt = 0; attempt < 3; ++attempt) {
-    if (attempt > 0 && (wc_hint > 0 || wc_try[attempt] >= a->W)) continue;
-    SlabParams q;
-    if (!slab_geometry(a, &q, wc_try[attempt])) { if (attempt == 0) break; else continue; }
-    if (attempt > 0 && q.wchunks == 1) continue;
-    int bn_c = 0, mt_c = 0, r_c = 0; bool flex_c = false;
-    const double cost = slab_pick_tiles(a, q, &bn_c, &flex_c, &mt_c, &r_c);
-    if (mt_c == 0) continue;
-    if (best_mt == 0 || cost < best_cost) { best_p = q; BN = bn_c; flex = flex_c; best_mt = mt_c; best_R = r_c; best_cost = cost; }
-  }
-  out[0] = best_mt != 0; out[1] = BN; out[2] = best_mt; out[3] = best_R; out[4] = best_p.PW; out[5] = best_p.WC; out[6] = best_p.wchunks;
-  const long long tq = best_mt ? (best_p.P + best_mt * 128 - 1) / (best_mt * 128) : 0;
-  out[7] = (int)(((a->ldy + BN - 1) / (BN ? BN : 1)) * tq * best_p.wchunks * a->N * best_p.To);
-  out[8] = flex; out[9] = remapped;
-  return B2_OK;
-}
-/* debug knobs of the small-M path: layers with M <= maxm take the dense-M kernel (0 = never); force_s > 0 caps the cluster size */
-int b2_debug_set_slab_wide(int on) { g_slab_wide = on; return B2_OK; }   /* -1 rule, 0 never, 1 always */
-/* host-only view of the temporal stack kernel's decision for a convolution (no launch, no GPU needed): out = {applies, items, frame
-   groups per clip, position tiles per frame, channel chunks, resident filter bytes, dynamic shared memory bytes} */
-int b2_debug_tstack_plan(const b2_conv_args* a, int* out) {
-  if (g_tstack == -2) { const char* e = getenv("B2_TSTACK"); g_tstack = (e && e[0] == '0') ? 0 : -1; }
-  TstackParams p;
-  size_t smem = 0;
-  memset(&p, 0, sizeof(p));
-  const bool ok = g_tstack != 0 && tstack_plan(a, &p, &smem);
-  out[0] = ok; out[1] = ok ? p.items_total : 0; out[2] = p.groups; out[3] = p.tiles_q; out[4] = p.cchunks;
-  out[5] = ok ? p.cchunks * p.kt * kTkWBlock : 0; out[6] = ok ? (int)smem : 0;
-  return B2_OK;
-}
-int b2_debug_last_conv_path(void) { return g_last_conv_path; }   /* 1: the temporal stack kernel took the last convolution */
-int b2_debug_set_tstack(int mode) { g_tstack = mode < -1 ? -1 : (mode > 1 ? 1 : mode); return B2_OK; }   /* temporal stack kernel: -1 rule, 0 never, 1 whenever eligible */
-int b2_debug_set_slab_mt(int mt) { g_slab_force_mt = mt < 0 ? 0 : mt; return B2_OK; }
-int b2_debug_set_densem(int maxm, int force_s) { g_densem_maxm = maxm < 0 ? -2 : maxm; g_densem_force_s = force_s; return B2_OK; }
-const char* b2_last_error(void) { return g_err; }
-uint64_t b2_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
-
-static int conv_out_dim(int in, int k, int s, int p) { return (in + 2 * p - k) / s + 1; }
 
 static int validate_conv(const b2_conv_args* a) {
   B2_CHECK_ARG(a != nullptr, "null args");
@@ -937,105 +863,12 @@ static int validate_conv(const b2_conv_args* a) {
   return B2_OK;
 }
 
-int b2_conv_ndhwc_fprop(const b2_conv_args* a, void* stream) {
-  int rc = validate_conv(a);
-  if (rc != B2_OK) return rc;
-  if ((rc = require_sm100()) != B2_OK) return rc;
-  const long long M_out = (long long)a->N * conv_out_dim(a->T, a->kt, a->st, a->pt) * conv_out_dim(a->H, a->kh, a->sh, a->ph) *
-                          conv_out_dim(a->W, a->kw, a->sw, a->pw);
-  const bool small_m = a->mode == B2_CONV_AUTO && !a->upsample && !a->aff_ld && !a->out_f32 && !a->y2 && !a->residual_up &&
-                       !a->residual_pre && !a->in_scale && g_gemm_algo == 0 &&
-                       densem_wanted(M_out, a->kt * a->kh * a->kw, a->st > 1 || a->sh > 1 || a->sw > 1);
-  g_last_conv_path = 0;
-  rc = small_m ? 0 : try_tstack(a, reinterpret_cast<cudaStream_t>(stream));
-  if (rc != 0) return rc < 0 ? rc : B2_OK;
-  rc = small_m ? 0 : try_slabts(a, reinterpret_cast<cudaStream_t>(stream));
-  if (rc != 0) return rc < 0 ? rc : B2_OK;
-  rc = small_m ? 0 : try_slab(a, reinterpret_cast<cudaStream_t>(stream));
-  if (rc != 0) return rc < 0 ? rc : B2_OK;
-  if (a->upsample) return set_error(B2_ERR_UNSUPPORTED, "fused upsampling needs the slab kernel, which does not take this shape");
-
-  IgemmLaunch L;
-  memset(&L, 0, sizeof(L));
-  IgemmParams& p = L.p;
-  p.x = reinterpret_cast<const __half*>(a->x);
-  p.N = a->N; p.T = a->T; p.H = a->H; p.W = a->W; p.C = a->C;
-  p.To = conv_out_dim(a->T, a->kt, a->st, a->pt);
-  p.Ho = conv_out_dim(a->H, a->kh, a->sh, a->ph);
-  p.Wo = conv_out_dim(a->W, a->kw, a->sw, a->pw);
-  p.kt = a->kt; p.kh = a->kh; p.kw = a->kw;
-  p.st = a->st; p.sh = a->sh; p.sw = a->sw;
-  p.pt = a->pt; p.ph = a->ph; p.pw = a->pw;
-  const long long M = (long long)a->N * p.To * p.Ho * p.Wo;
-  B2_CHECK_ARG(M < (1ll << 31), "output too large");
-  p.M_total = (int)M;
-  p.Ncols = a->K;
-  p.scale = a->scale; p.shift = a->shift;
-  p.residual = reinterpret_cast<const __half*>(a->residual);
-  p.ldr = a->ldr;
-  p.y = a->y; p.ldy = a->ldy;
-  p.relu = a->relu; p.per_row = 0; p.accumulate = a->accumulate;
-  p.epi = a->out_f32 ? EPI_DIRECT_F32 : EPI_TMA_F16;
-  p.aff_ld = a->aff_ld;
-  p.res_up = a->residual_up; p.res_pre = a->residual_pre; p.up_H = p.Ho; p.up_W = p.Wo;
-  p.y2 = a->y2; p.scale2 = a->scale2; p.shift2 = a->shift2; p.aff2_ld = a->aff2_ld; p.aff2_rows = p.To * p.Ho * p.Wo;
-  if (a->y2) {
-    B2_CHECK_ARG(a->scale2 && a->shift2 && a->aff2_ld >= a->K && !a->out_f32 && a->kt * a->kh * a->kw == 1,
-                 "second output needs scale2 / shift2 (fp32 [N][aff2_ld >= K]) and a 1x1 convolution with fp16 output");
-    if (p.aff2_rows % 128 != 0)
-      return set_error(B2_ERR_UNSUPPORTED, "second output with a per-sample affine needs To*Ho*Wo %% 128 == 0 (got %d)", p.aff2_rows);
+static int validate_gemm(const b2_gemm_args* g, bool pair, const void* a2, int lda2, const void* b2, int ldb2, int k2) {
+  if (pair) {        // b2_gemm2_f16
+    B2_CHECK_ARG(g != nullptr && a2 && b2 && k2 > 0, "null / empty second operand pair");
+    B2_CHECK_ARG(lda2 % 8 == 0 && ldb2 % 8 == 0 && lda2 >= k2 && ldb2 >= k2, "bad second operand pitch");
+    B2_CHECK_ARG(!g->out_f32 && !g->per_row, "the fused two-operand GEMM produces fp16 output with per-column affine");
   }
-  if (a->in_scale) {
-    B2_CHECK_ARG(a->in_shift && a->in_aff_ld >= a->C && (a->in_aff_ld & 3) == 0 && !a->out_f32 && a->kt * a->kh * a->kw == 1 && a->st == 1 &&
-                     a->sh == 1 && a->sw == 1 && (reinterpret_cast<uintptr_t>(a->in_scale) & 15) == 0 &&
-                     (reinterpret_cast<uintptr_t>(a->in_shift) & 15) == 0,
-                 "input affine needs in_shift, a 16-byte aligned fp32 [N][in_aff_ld >= C] pair (pitch %% 4 == 0) and a 1x1 stride-1 convolution with fp16 output");
-    if ((p.To * p.Ho * p.Wo) % 128 != 0 || a->C % 64 != 0)
-      return set_error(B2_ERR_UNSUPPORTED, "input affine needs To*Ho*Wo %% 128 == 0 and a channel pitch that is a multiple of 64 (got %d, %d)",
-                       p.To * p.Ho * p.Wo, a->C);
-    p.in_scale = a->in_scale; p.in_shift = a->in_shift; p.in_ld = a->in_aff_ld; p.in_rows = p.To * p.Ho * p.Wo;
-  }
-  p.aff_rows = p.To * p.Ho * p.Wo;
-  if (a->aff_ld && p.aff_rows % 128 != 0)
-    return set_error(B2_ERR_UNSUPPORTED, "per-sample affine on a 1x1x1 convolution needs To*Ho*Wo %% 128 == 0 (got %d)", p.aff_rows);
-  L.w = a->w;
-
-  const int taps = a->kt * a->kh * a->kw;
-  if (a->mode == B2_CONV_STEM7) {
-    B2_CHECK_ARG(!a->out_f32 && a->residual == nullptr, "stem convolution has no residual / fp32 output");
-    B2_CHECK_ARG(a->st == 1 && a->sh == 2, "stem convolution needs strides (1, 2, 2)");
-    const cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    return a->K <= 64 ? launch_stem<64>(a, st) : launch_stem<128>(a, st);
-  } else if (taps == 1 && a->st == 1 && a->sh == 1 && a->sw == 1 && a->pt == 0 && a->ph == 0 && a->pw == 0) {
-    // 1x1x1 stride-1: A is literally the [M][C] activation matrix -> TMA on both operands
-    p.amode = AMODE_TMA;
-    p.nkb = (a->C + kBK - 1) / kBK;
-    L.a_mat = a->x; L.lda = a->C; L.a_cols = a->C;
-    L.ldb = a->C; L.b_cols = a->C;
-  } else {
-    p.amode = AMODE_GATHER;
-    p.cchunks = (a->C + kBK - 1) / kBK;
-    p.nkb = taps * p.cchunks;
-    L.ldb = taps * a->C;
-    L.b_cols = L.ldb;
-    // When C % 64 != 0 the last K block of a tap also covers the first columns of the next tap's
-    // weights; the activation side zero-fills channels >= C, so those products vanish.
-  }
-  return dispatch_igemm(L, reinterpret_cast<cudaStream_t>(stream));
-}
-
-static int gemm_common(const b2_gemm_args* g, const void* a2, int lda2, const void* b2, int ldb2, int k2, void* stream);
-
-int b2_gemm_f16(const b2_gemm_args* g, void* stream) { return gemm_common(g, nullptr, 0, nullptr, 0, 0, stream); }
-
-int b2_gemm2_f16(const b2_gemm_args* g, const void* a2, int lda2, const void* b2, int ldb2, int k2, void* stream) {
-  B2_CHECK_ARG(g != nullptr && a2 && b2 && k2 > 0, "null / empty second operand pair");
-  B2_CHECK_ARG(lda2 % 8 == 0 && ldb2 % 8 == 0 && lda2 >= k2 && ldb2 >= k2, "bad second operand pitch");
-  B2_CHECK_ARG(!g->out_f32 && !g->per_row, "the fused two-operand GEMM produces fp16 output with per-column affine");
-  return gemm_common(g, a2, lda2, b2, ldb2, k2, stream);
-}
-
-static int gemm_common(const b2_gemm_args* g, const void* a2, int lda2, const void* b2, int ldb2, int k2, void* stream) {
   B2_CHECK_ARG(g != nullptr, "null args");
   B2_CHECK_ARG(g->a && g->b && g->scale && g->shift && g->d, "null tensor pointer");
   B2_CHECK_ARG(g->M > 0 && g->N > 0 && g->Kd > 0, "non-positive dimension");
@@ -1046,37 +879,70 @@ static int gemm_common(const b2_gemm_args* g, const void* a2, int lda2, const vo
     B2_CHECK_ARG(!g->accumulate, "accumulate requires out_f32");
     B2_CHECK_ARG(g->residual == nullptr || (g->ldr % 8 == 0 && g->ldr >= g->N), "bad residual pitch");
   }
-  int rc;
-  if ((rc = require_sm100()) != B2_OK) return rc;
-
-  IgemmLaunch L;
-  memset(&L, 0, sizeof(L));
-  IgemmParams& p = L.p;
-  p.amode = AMODE_TMA;
-  p.M_total = g->M;
-  p.Ncols = g->N;
-  p.nkb = (g->Kd + kBK - 1) / kBK;
-  p.scale = g->scale; p.shift = g->shift;
-  p.residual = reinterpret_cast<const __half*>(g->residual);
-  p.ldr = g->ldr;
-  p.y = g->d; p.ldy = g->ldd;
-  p.relu = g->relu; p.per_row = g->per_row; p.accumulate = g->accumulate;
-  p.epi = g->out_f32 ? EPI_DIRECT_F32 : EPI_TMA_F16;
-  B2_CHECK_ARG(g->aff_ld >= 0 && (g->aff_ld == 0 || (g->aff_ld >= g->N && g->aff_rows > 0 && g->aff_rows % 128 == 0 &&
-                                                     !g->out_f32 && !g->per_row)),
-               "bad per-sample affine (pitch %d, rows per sample %d)", g->aff_ld, g->aff_rows);
-  p.aff_ld = g->aff_ld; p.aff_rows = g->aff_rows;
-  if (g->d2) {
-    B2_CHECK_ARG(g->scale2 && g->shift2 && g->aff2_ld >= g->N && g->aff2_rows > 0 && g->aff2_rows % 128 == 0 && !g->out_f32 && !g->per_row,
-                 "second output needs scale2 / shift2 (fp32 [M / aff2_rows][aff2_ld >= N], aff2_rows %% 128 == 0) and fp16 output");
-    p.y2 = g->d2; p.scale2 = g->scale2; p.shift2 = g->shift2; p.aff2_ld = g->aff2_ld; p.aff2_rows = g->aff2_rows;
-  }
-  p.x = reinterpret_cast<const __half*>(g->a);
-  L.a_mat = g->a; L.lda = g->lda; L.a_cols = g->Kd;
-  L.w = g->b; L.ldb = g->ldb; L.b_cols = g->Kd;
-  L.a2 = a2; L.lda2 = lda2; L.w2 = b2; L.ldb2 = ldb2; L.k2 = k2;
-  if (k2 > 0 && g_gemm_algo != 0) return set_error(B2_ERR_UNSUPPORTED, "two-operand GEMM needs the persistent kernel");
-  return dispatch_igemm(L, reinterpret_cast<cudaStream_t>(stream));
+  return B2_OK;
 }
+
+static int run_gemm(bool pair, const b2_gemm_args* g, const void* a2, int lda2, const void* b2, int ldb2, int k2, void* stream) {
+  ConvPlan pl;
+  B2_TRY(validate_gemm(g, pair, a2, lda2, b2, ldb2, k2));
+  B2_TRY(require_sm100());
+  B2_TRY(plan_gemm(g, a2, lda2, b2, ldb2, k2, &pl));
+  return launch_plan(pl, reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" {
+
+int b2_version(void) { return 103; }   // 103: split-K / fused (2+1)D / pooled-stem entry points (round 2); 102: generator fields
+
+int b2_conv_ndhwc_fprop(const b2_conv_args* a, void* stream) {
+  ConvPlan pl;
+  g_last_conv_kernel = KERN_NONE;
+  B2_TRY(validate_conv(a));
+  B2_TRY(require_sm100());
+  B2_TRY(plan_conv(a, &pl));
+  B2_TRY(launch_plan(pl, reinterpret_cast<cudaStream_t>(stream)));
+  g_last_conv_kernel = pl.kernel;
+  return B2_OK;
+}
+
+int b2_gemm_f16(const b2_gemm_args* g, void* stream) { return run_gemm(false, g, nullptr, 0, nullptr, 0, 0, stream); }
+
+int b2_gemm2_f16(const b2_gemm_args* g, const void* a2, int lda2, const void* b2, int ldb2, int k2, void* stream) {
+  return run_gemm(true, g, a2, lda2, b2, ldb2, k2, stream);
+}
+
+/* Debug entry points (not in the public header).  The *_plan probes validate and plan a call exactly as the entry point would,
+   without a launch or a device: out[0 .. n) = the plan_view fields (kernel id as in enum ConvKernel, grid, block, dynamic shared
+   memory, cluster size, then the kernel's tiling).  Without a device sm_count() is 148, the B200's, so these are B200 plans. */
+int b2_debug_conv_plan(const b2_conv_args* a, int* out, int n) {
+  ConvPlan pl;
+  B2_TRY(validate_conv(a));
+  B2_TRY(plan_conv(a, &pl));
+  return plan_view(pl, a->kt, out, n);
+}
+/* k2 > 0: the two-operand GEMM of b2_gemm2_f16, with the second pair at the first pair's addresses and pitch round_up(k2, 8) */
+int b2_debug_gemm_plan(const b2_gemm_args* g, int k2, int* out, int n) {
+  ConvPlan pl;
+  const int ld2 = (k2 + 7) / 8 * 8;
+  const void* a2 = k2 > 0 && g ? g->a : nullptr;
+  const void* b2 = k2 > 0 && g ? g->b : nullptr;
+  B2_TRY(validate_gemm(g, k2 > 0, a2, ld2, b2, ld2, k2));
+  B2_TRY(plan_gemm(g, a2, ld2, b2, ld2, k2, &pl));
+  return plan_view(pl, 1, out, n);
+}
+int b2_debug_last_conv_kernel(void) { return g_last_conv_kernel; }
+int b2_debug_last_conv_path(void) { return g_last_conv_kernel == KERN_TSTACK; }   /* 1: the temporal stack kernel took it */
+/* 0 = auto, 1 = no slab / temporal-group / temporal stack kernels */
+int b2_debug_set_conv_algo(int algo) {
+  if (algo != 0 && algo != 1) return set_error(B2_ERR_INVALID, "conv algo %d: 0 (auto) or 1 (gather)", algo);
+  tuning().conv_algo = algo;
+  return B2_OK;
+}
+int b2_debug_set_gemm_algo(int algo) { tuning().gemm_algo = algo; return B2_OK; }
+int b2_debug_set_slab_wide(int on) { tuning().slab_wide = on; return B2_OK; }   /* -1 rule, 0 never, 1 always */
+int b2_debug_set_tstack(int mode) { tuning().tstack = mode < -1 ? -1 : (mode > 1 ? 1 : mode); return B2_OK; }   /* -1 rule, 0 never, 1 whenever eligible */
+int b2_debug_set_slab_mt(int mt) { tuning().slab_mt = mt < 0 ? 0 : mt; return B2_OK; }
+/* small-M path: layers with M <= maxm take the dense-M kernel (0 = never, < 0 = the rule); force_s > 0 caps the cluster size */
+int b2_debug_set_densem(int maxm, int force_s) { tuning().densem_maxm = maxm < 0 ? -1 : maxm; tuning().densem_s = force_s; return B2_OK; }
 
 }  // extern "C"

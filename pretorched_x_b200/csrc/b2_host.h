@@ -1,4 +1,4 @@
-// b2_host.h -- host-side helpers shared by the C-ABI translation units: error reporting, launch
+// b2_host.h -- host-side helpers shared by the C-ABI translation units (defined in b2_host.cu): error reporting, launch
 // accounting and CUtensorMap construction through the driver entry point (no -lcuda link needed).
 #pragma once
 
@@ -22,6 +22,12 @@ void count_launch(int n = 1);
     if (!(cond)) return ::b2::set_error(B2_ERR_INVALID, __VA_ARGS__); \
   } while (0)
 
+#define B2_TRY(expr)                              \
+  do {                                            \
+    const int rc__ = (expr);                      \
+    if (rc__ != B2_OK) return rc__;               \
+  } while (0)
+
 #define B2_CHECK_CUDA(expr)                                                                         \
   do {                                                                                              \
     cudaError_t e__ = (expr);                                                                       \
@@ -43,7 +49,7 @@ void count_launch(int n = 1);
 // GPUs (nn.DataParallel -- the reference's only multi-GPU construct -- or model.to('cuda:1')) must opt in on each of them.
 // One bit per device ordinal, set after the first successful call on that device.
 int current_device();
-int sm_count();          // SM count of the current device (cached per ordinal)
+int sm_count();          // SM count of the current device (cached per ordinal); 148, the B200's, when there is no device
 #define B2_OPT_IN_SMEM(kernel, bytes)                                                                          \
   do {                                                                                                         \
     static std::atomic<unsigned long long> done__{0};                                                          \
@@ -54,16 +60,32 @@ int sm_count();          // SM count of the current device (cached per ordinal)
     }                                                                                                          \
   } while (0)
 
+// A CUtensorMap as plain values: what cuTensorMapEncodeTiled takes (strides in bytes, for dims 1 .. rank-1).  The builders
+// below check what can be checked on the host (alignment, pitch, box limits) and fill one; encode_tmap makes the map.
+struct TmapSpec {
+  const void* base;
+  CUtensorMapDataType dtype;
+  int rank;
+  cuuint64_t dims[4];
+  cuuint64_t strides[3];
+  cuuint32_t box[4];
+  cuuint32_t estr[4];
+  bool swizzle128;
+};
+int encode_tmap(CUtensorMap* out, const TmapSpec& spec);
+
 // 2-D fp16 tensor map: `inner` contiguous elements per row, `outer` rows of pitch `pitch_elems`;
 // box = [box_inner x box_outer]; swizzle128 selects CU_TENSOR_MAP_SWIZZLE_128B (box_inner must be 64).
 // Out-of-bounds elements read as zero and are dropped on store.
+int tmap_2d_f16(TmapSpec* out, const void* base, uint64_t inner, uint64_t outer, uint64_t pitch_elems, uint32_t box_inner,
+                uint32_t box_outer, bool swizzle128);
 int make_tmap_2d_f16(CUtensorMap* out, const void* base, uint64_t inner, uint64_t outer, uint64_t pitch_elems,
                      uint32_t box_inner, uint32_t box_outer, bool swizzle128);
 
-// 4-D fp16 tensor map over an NDHWC activation viewed as (C, W, H, N*T); smem box = (64, box_w, box_h, 1) pixels
+// 4-D fp16 tensor map over an NDHWC activation viewed as (C, W, H, N*T); smem box = (64, box_w, box_h, box_planes) pixels
 // taken every stride_hw-th column / row (TMA elementStrides), SWIZZLE_128B.  Negative / out-of-range box coordinates read zeros (halo columns, rows above/below the image).
-int make_tmap_ndhwc_slab(CUtensorMap* out, const void* base, uint64_t C, uint64_t W, uint64_t H, uint64_t planes,
-                         uint32_t box_w, uint32_t box_h, uint32_t stride_hw, uint32_t box_planes = 1);
+int tmap_ndhwc_slab(TmapSpec* out, const void* base, uint64_t C, uint64_t W, uint64_t H, uint64_t planes, uint32_t box_w,
+                    uint32_t box_h, uint32_t stride_hw, uint32_t box_planes = 1);
 
 int require_sm100();
 

@@ -1,6 +1,9 @@
 """GPU (-m gpu): kernel-level parity of the C-ABI entry points against the CPU oracle (torch fp32 on the same
 fp16-rounded operands).  Tolerances are relative to max|reference|: 2e-3 for fp16 outputs (fp32 accumulate,
 one fp16 rounding of the result = 2^-11), 1e-4 for fp32 outputs."""
+import functools
+import json
+import os
 import zlib
 
 import pytest
@@ -34,6 +37,14 @@ def rel(got, ref):
 
 def seed_of(name):
     return zlib.crc32(name.encode()) % 100000
+
+
+@functools.lru_cache(maxsize=None)
+def golden_kernels():
+    """Case name -> the kernel instance its convolution launched on the B200 that recorded tests/golden/conv_plans.json."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "conv_plans.json")) as fh:
+        rows = json.load(fh)["rows"]
+    return {src.split(":", 1)[1]: r["kernel"] for r in rows for src in r["sources"] if src.startswith(("conv_case:", "tstack_case:"))}
 
 
 CONV_CASES = [
@@ -160,6 +171,9 @@ def check_conv_case(dev, case, simt):
     a = ops.from_ncdhw(x.to(dev))
     ra = ops.from_ncdhw(r.to(dev), pitch=ops._round_up(K, 8)) if res else None
     out = engine.conv_bn_act(conv.to(dev), bnm.to(dev) if bnm is not None else None, a, residual=ra, relu=relu, simt=simt)
+    if not simt and name in golden_kernels():              # the case ran on the kernel its name is about
+        from pretorched_x_b200 import _lib
+        assert _lib.last_conv_kernel() == golden_kernels()[name]
     assert (out.N, out.T, out.H, out.W, out.C) == (y.shape[0], y.shape[2], y.shape[3], y.shape[4], K)
     assert rel(ops.to_ncdhw(out), y) <= TOL_F16
     if out.ld > out.C:                                     # channel padding must stay exactly zero

@@ -123,74 +123,60 @@ def test_shard_bounds_cover_batch_exactly():
             assert max(sizes) - min(sizes) <= 1
 
 
-def test_slab_tiling_plan_is_host_logic():
-    """The slab kernel's tiling decision (N tile, M tiles per item, slab rows, W chunking) is pure host code behind a debug entry
-    point: the shapes of the BASELINE nets must be accepted with a plan that fits TMEM (MT * N <= 512 columns)."""
-    import ctypes
+def _conv_plan(N, C, T, H, W, K, k, s=(1, 1, 1), pad=None):
+    """The plan b2_conv_ndhwc_fprop would launch for a BN + ReLU convolution of these dimensions (host code, no GPU needed)."""
     from pretorched_x_b200 import _lib
-    lib = _lib.load()
-    lib.b2_debug_slab_plan.argtypes = [ctypes.POINTER(_lib.ConvArgs), ctypes.POINTER(ctypes.c_int)]
+    a = _lib.ConvArgs()
+    a.x = a.w = a.scale = a.shift = a.y = 1 << 20               # never dereferenced: the probe plans, it does not launch
+    a.N, a.T, a.H, a.W, a.C, a.K = N, T, H, W, (C + 7) // 8 * 8, K
+    a.ldy = (K + 7) // 8 * 8
+    a.kt, a.kh, a.kw = k
+    a.st, a.sh, a.sw = s
+    a.pt, a.ph, a.pw = pad if pad is not None else (k[0] // 2, k[1] // 2, k[2] // 2)
+    return _lib.conv_plan(a)
 
-    def plan(N, C, T, H, W, K, k, s=(1, 1, 1)):
-        a = _lib.ConvArgs()
-        a.N, a.T, a.H, a.W, a.C, a.K = N, T, H, W, (C + 7) // 8 * 8, K
-        a.ldy = (K + 7) // 8 * 8
-        a.kt, a.kh, a.kw = k
-        a.st, a.sh, a.sw = s
-        a.pt, a.ph, a.pw = k[0] // 2, k[1] // 2, k[2] // 2
-        out = (ctypes.c_int * 10)()
-        assert lib.b2_debug_slab_plan(ctypes.byref(a), out) == 0
-        return dict(zip("applies BN MT R PW WC wchunks items flex remap".split(), list(out)))
 
-    p = plan(32, 64, 8, 56, 56, 64, (3, 3, 3))                     # resnet3d50 layer1 conv2
-    assert p["applies"] and p["BN"] == 64 and 1 <= p["MT"] <= 4 and p["PW"] == 58 and p["wchunks"] == 1
+def test_conv_plan_slab_tiling():
+    """The slab kernels' tiling decision (N tile, M tiles per item, slab rows, W chunking) is pure host code behind a debug entry
+    point: the shapes of the BASELINE nets must be accepted with a plan that fits TMEM (MT * N <= 512 columns)."""
+    plan = _conv_plan
+    p = plan(32, 64, 8, 56, 56, 64, (3, 3, 3))                     # resnet3d50 layer1 conv2: the temporal-group slab kernel
+    assert p["kernel"] == "slabts" and p["bn"] == 64 and 1 <= p["MT"] <= 4 and p["PW"] == 58 and p["wchunks"] == 1
     p = plan(16, 64, 16, 28, 28, 144, (1, 3, 3))                   # R(2+1)D layer1 spatial: runtime N tile of 144 columns
-    assert p["applies"] and p["flex"] and p["BN"] == 144 and p["MT"] * 160 <= 512
-    p = plan(16, 144, 16, 28, 28, 64, (3, 1, 1))                   # temporal conv: remapped to frames x positions, 64-wide chunks
-    assert p["applies"] and p["remap"] and p["WC"] <= 64 and p["wchunks"] >= 13
+    assert p["kernel"] == "slab<0>" and p["flex"] and p["bn"] == 144 and p["MT"] * 160 <= 512
+    p = plan(2, 144, 16, 28, 28, 64, (3, 1, 1))                    # temporal conv: remapped to frames x positions, 64-wide chunks
+    assert p["kernel"] == "slab<64>" and p["remap"] and p["WC"] <= 64 and p["wchunks"] >= 13
+    assert plan(16, 144, 16, 28, 28, 64, (3, 1, 1))["kernel"] == "tstack"   # its BASELINE-batch twin: the temporal stack kernel
     p = plan(1, 64, 1, 6, 300, 64, (1, 3, 3))                      # rows longer than a TMA box are cut into W chunks
-    assert p["applies"] and p["wchunks"] >= 2 and p["PW"] <= 256
-    assert not plan(2, 64, 4, 8, 8, 256, (1, 1, 1))["applies"]     # 1x1x1: persistent GEMM, not the slab kernel
+    assert p["kernel"] == "slab<64>" and p["wchunks"] >= 2 and p["PW"] <= 256
+    assert plan(2, 64, 4, 8, 8, 256, (1, 1, 1))["kernel"] == "pgemm<128,0>"   # 1x1x1: persistent GEMM, not the slab kernel
 
 
-def test_temporal_stack_plan_is_host_logic():
+def test_conv_plan_temporal_stack():
     """Which convolutions the temporal stack kernel (b2_tstack.cuh) takes, and with what decomposition: pure host code behind a debug
     entry point.  The 64-wide temporal halves of R(2+1)D-34 at the BASELINE batch are taken with the filter resident; launches with
     less than one work item per SM, wider outputs, strided / spatial filters and filters too big to stay resident are not."""
-    import ctypes
     from pretorched_x_b200 import _lib
     lib = _lib.load()
-    lib.b2_debug_tstack_plan.argtypes = [ctypes.POINTER(_lib.ConvArgs), ctypes.POINTER(ctypes.c_int)]
-
-    def plan(N, C, T, H, W, K, k, s=(1, 1, 1), pad=None):
-        a = _lib.ConvArgs()
-        a.N, a.T, a.H, a.W, a.C, a.K = N, T, H, W, (C + 7) // 8 * 8, K
-        a.ldy = (K + 7) // 8 * 8
-        a.kt, a.kh, a.kw = k
-        a.st, a.sh, a.sw = s
-        a.pt, a.ph, a.pw = pad if pad is not None else (k[0] // 2, k[1] // 2, k[2] // 2)
-        out = (ctypes.c_int * 7)()
-        assert lib.b2_debug_tstack_plan(ctypes.byref(a), out) == 0
-        return dict(zip("applies items groups tiles cchunks wbytes smem".split(), list(out)))
-
+    plan = _conv_plan
     lib.b2_debug_set_tstack(-1)
     p = plan(16, 110, 32, 56, 56, 64, (7, 1, 1))                   # R(2+1)D stem, temporal half: 8 groups of 4 frames x 25 tiles x 16 clips
-    assert p["applies"] and (p["items"], p["groups"], p["tiles"], p["cchunks"]) == (3200, 8, 25, 2)
+    assert p["kernel"] == "tstack" and (p["items"], p["groups"], p["tiles"], p["cchunks"]) == (3200, 8, 25, 2)
     assert p["wbytes"] == 2 * 7 * 8192 and p["smem"] <= 227 * 1024
     p = plan(16, 144, 16, 28, 28, 64, (3, 1, 1))                   # layer1 temporal halves: 3 channel chunks, 72 KB filter
-    assert p["applies"] and (p["items"], p["groups"], p["tiles"], p["cchunks"], p["wbytes"]) == (448, 4, 7, 3, 73728)
-    assert not plan(2, 144, 16, 28, 28, 64, (3, 1, 1))["applies"]   # 56 items < one per SM: the slab kernel keeps more SMs busy
-    assert not plan(16, 288, 8, 14, 14, 128, (3, 1, 1))["applies"]  # 128 output channels: N = 128 MMAs are balanced already
-    assert not plan(16, 64, 16, 28, 28, 64, (3, 3, 3))["applies"]   # in-plane taps: slab / slabts
-    assert not plan(16, 230, 8, 14, 14, 64, (3, 1, 1), s=(2, 1, 1))["applies"]   # temporal stride
-    assert not plan(16, 64, 16, 28, 28, 64, (3, 1, 1), pad=(0, 0, 0))["applies"]  # not "same"-padded
-    assert not plan(64, 1024, 8, 14, 14, 64, (3, 1, 1))["applies"]  # 16 chunks x 3 taps x 8 KB = 384 KB: cannot stay resident
-    assert not plan(64, 64, 1, 56, 56, 64, (3, 1, 1))["applies"]    # a single frame: only the centre tap ever sees data
+    assert p["kernel"] == "tstack" and (p["items"], p["groups"], p["tiles"], p["cchunks"], p["wbytes"]) == (448, 4, 7, 3, 73728)
+    assert plan(2, 144, 16, 28, 28, 64, (3, 1, 1))["kernel"] == "slab<64>"     # 56 items < one per SM: the slab kernel keeps more SMs busy
+    assert plan(16, 288, 8, 14, 14, 128, (3, 1, 1))["kernel"] == "slab<128>"   # 128 output channels: N = 128 MMAs are balanced already
+    assert plan(16, 64, 16, 28, 28, 64, (3, 3, 3))["kernel"] == "slabts"       # in-plane taps: slab / slabts
+    assert plan(16, 230, 8, 14, 14, 64, (3, 1, 1), s=(2, 1, 1))["kernel"] == "slab<64>"    # temporal stride
+    assert plan(16, 64, 16, 28, 28, 64, (3, 1, 1), pad=(0, 0, 0))["kernel"] == "igemm<64>"  # not "same"-padded
+    assert plan(64, 1024, 8, 14, 14, 64, (3, 1, 1))["kernel"] == "slab<64>"    # 16 chunks x 3 taps x 8 KB = 384 KB: cannot stay resident
+    assert plan(64, 64, 1, 56, 56, 64, (3, 1, 1))["kernel"] == "slab<64>"      # a single frame: only the centre tap ever sees data
     try:
         lib.b2_debug_set_tstack(1)                                 # forced (tests): eligibility without the one-item-per-SM rule
-        assert plan(2, 144, 16, 28, 28, 64, (3, 1, 1))["applies"]
+        assert plan(2, 144, 16, 28, 28, 64, (3, 1, 1))["kernel"] == "tstack"
         lib.b2_debug_set_tstack(0)
-        assert not plan(16, 110, 32, 56, 56, 64, (7, 1, 1))["applies"]
+        assert plan(16, 110, 32, 56, 56, 64, (7, 1, 1))["kernel"] == "slab<64>"
     finally:
         lib.b2_debug_set_tstack(-1)
 
