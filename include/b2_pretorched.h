@@ -250,6 +250,39 @@ int b2_rgb_head_gather_tanh(const void* partial, int ldp, const float* bias, voi
 /* y[n][c][s] = tanh(x[n*S + s][c]): fp16 channels-last (pitch ldx) -> NCHW planes, fp32 (out_f32) or fp16. */
 int b2_tanh_nhwc_to_nchw(const void* x, int ldx, void* y, int N, int C, long long S, int out_f32, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Backward of the residual blocks with frozen BatchNorm statistics (fine-tuning of the last stages, b2_train.cu).
+ * ------------------------------------------------------------------------------------------- */
+/* gz[r][c] = (y[r][c] > 0) ? g[r][c] : 0 over M rows of pitch ldy (g: pitch ldg >= ldy), fp16; sum[c] = sum_r gz[r][c] in
+ * fp32 for c < ldy.  partial: fp32 scratch of b2_relu_grad_sum_partials(M, ldy) * ldy floats.  The sums are reduced in a
+ * fixed order (per-block partials, then the blocks in order): two calls give bit-identical results.  ldy <= 2048. */
+int b2_relu_grad_sum_partials(long long M, int ld);
+int b2_relu_grad_sum(const void* y, int ldy, const void* g, int ldg, void* gz, long long M, float* partial, float* sum,
+                     void* stream);
+/* y [N][T][H][W][ld] = g at the positions (s*to, s*ho, s*wo) and zero elsewhere; g has the stride-s output geometry
+ * (floor((T - 1) / s) + 1, ...) and pitch ld.  The data gradient of a stride-s, k = 2p + 1 convolution is the stride-1
+ * convolution of y with the flipped, transposed filter. */
+int b2_zero_dilate_scatter(const void* g, void* y, int N, int T, int H, int W, int ld, int stride, void* stream);
+/* y[n, s*to, s*ho, s*wo, c] += g[n, to, ho, wo, c] for c < C (fp32 add, fp16 store): the data gradient of a stride-s
+ * subsampling (the type-A shortcut, the strided 1x1x1 projection).  y: [N][T][H][W] pitch ldy; g: the subsampled
+ * geometry, pitch ldg. */
+int b2_strided_scatter_add(const void* g, int ldg, void* y, int ldy, int N, int T, int H, int W, int C, int stride, void* stream);
+/* Weight gradient of a convolution as an implicit GEMM on tcgen05, read straight from the two activation matrices:
+ *     dw[k][tap][c] = sum over output positions p of g[p][k] * x[p * stride + tap - pad][c]   (fp32, [K][taps][C])
+ * x: fp16 NDHWC [N][T][H][W], pitch ldx; g: fp16 rows of the output geometry, pitch ldg; C a multiple of 64; sh == sw.
+ * When the plan splits the positions, `work` must hold b2_wgrad_workspace_floats() floats; the splits are summed in a
+ * fixed order, so two calls give bit-identical results. */
+typedef struct b2_wgrad_args {
+  const void* x;
+  const void* g;
+  float* dw;
+  float* work;
+  int32_t N, T, H, W, ldx, C, ldg, K;
+  int32_t kt, kh, kw, st, sh, sw, pt, ph, pw;
+} b2_wgrad_args;
+size_t b2_wgrad_workspace_floats(const b2_wgrad_args* a);
+int b2_conv_ndhwc_wgrad(const b2_wgrad_args* a, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -54,6 +54,16 @@ class GemmArgs(ctypes.Structure):
     ]
 
 
+class WgradArgs(ctypes.Structure):
+    """Mirror of `struct b2_wgrad_args`."""
+    _fields_ = [
+        ("x", c_void_p), ("g", c_void_p), ("dw", c_void_p), ("work", c_void_p),
+        ("N", c_i32), ("T", c_i32), ("H", c_i32), ("W", c_i32), ("ldx", c_i32), ("C", c_i32), ("ldg", c_i32), ("K", c_i32),
+        ("kt", c_i32), ("kh", c_i32), ("kw", c_i32), ("st", c_i32), ("sh", c_i32), ("sw", c_i32),
+        ("pt", c_i32), ("ph", c_i32), ("pw", c_i32),
+    ]
+
+
 # name -> (restype, argtypes); every symbol include/b2_pretorched.h declares
 SYMBOLS = {
     "b2_version": (c_int, []),
@@ -85,6 +95,12 @@ SYMBOLS = {
     "b2_ccbn_act_ndhwc": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p] + [c_int] * 7 + [c_void_p]),
     "b2_rgb_head_gather_tanh": (c_int, [c_void_p, c_int, c_void_p, c_void_p] + [c_int] * 5 + [c_void_p]),
     "b2_tanh_nhwc_to_nchw": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, ctypes.c_longlong, c_int, c_void_p]),
+    "b2_relu_grad_sum_partials": (c_int, [ctypes.c_longlong, c_int]),
+    "b2_relu_grad_sum": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p]),
+    "b2_zero_dilate_scatter": (c_int, [c_void_p, c_void_p] + [c_int] * 6 + [c_void_p]),
+    "b2_wgrad_workspace_floats": (ctypes.c_size_t, [ctypes.POINTER(WgradArgs)]),
+    "b2_conv_ndhwc_wgrad": (c_int, [ctypes.POINTER(WgradArgs), c_void_p]),
+    "b2_strided_scatter_add": (c_int, [c_void_p, c_int, c_void_p, c_int] + [c_int] * 6 + [c_void_p]),
 }
 
 
@@ -116,6 +132,28 @@ def conv_plan(args):
 def gemm_plan(args, k2=0):
     """What b2_gemm_f16 (k2 == 0) or b2_gemm2_f16 (a second operand pair of depth k2) would launch for ``args`` (a GemmArgs)."""
     return _plan("b2_debug_gemm_plan", GemmArgs, args, k2)
+
+
+WGRAD_PLAN_FIELDS = ("grid_x", "grid_y", "block", "smem", "mt", "nt", "taps", "rects", "splits", "rect_cols", "rect_rows")
+
+
+def wgrad_plan(args):
+    """What b2_conv_ndhwc_wgrad would launch for ``args`` (a WgradArgs), as a dict of WGRAD_PLAN_FIELDS plus ``ranges``, the
+    position-rectangle range [r0, r1) of every split.  Host code only (148 SMs without a device)."""
+    lib = load()
+    fn, rng = lib.b2_debug_wgrad_plan, lib.b2_debug_wgrad_split
+    fn.restype, fn.argtypes = c_int, [ctypes.POINTER(WgradArgs), ctypes.POINTER(c_int), c_int]
+    rng.restype, rng.argtypes = c_int, [ctypes.POINTER(WgradArgs), c_int, ctypes.POINTER(ctypes.c_longlong)]
+    out = (c_int * len(WGRAD_PLAN_FIELDS))()
+    check(fn(ctypes.byref(args), out, len(WGRAD_PLAN_FIELDS)), "b2_debug_wgrad_plan")
+    plan = dict(zip(WGRAD_PLAN_FIELDS, out))
+    ranges = []
+    for s in range(plan["splits"]):
+        r = (ctypes.c_longlong * 2)()
+        check(rng(ctypes.byref(args), s, r), "b2_debug_wgrad_split")
+        ranges.append((r[0], r[1]))
+    plan["ranges"] = ranges
+    return plan
 
 
 def last_conv_kernel():

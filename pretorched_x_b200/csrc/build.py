@@ -12,7 +12,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["b2_host.cu", "b2_conv_api.cu", "b2_aux.cu", "b2_attention.cu", "b2_gan.cu", "b2_image.cu", "b2_probe.cu"]
+SOURCES = ["b2_host.cu", "b2_conv_api.cu", "b2_aux.cu", "b2_attention.cu", "b2_gan.cu", "b2_image.cu", "b2_probe.cu", "b2_train.cu"]
 HEADERS = ["b2_ptx.cuh", "b2_igemm.cuh", "b2_densem.cuh", "b2_pgemm.cuh", "b2_slabconv.cuh", "b2_slabts.cuh", "b2_tstack.cuh", "b2_stemconv.cuh",
            "b2_host.h", "../../include/b2_pretorched.h"]
 LIB = os.path.join(HERE, "libb2pretorched.so")

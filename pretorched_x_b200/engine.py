@@ -212,11 +212,15 @@ def run_bottleneck(block, a, simt=False, out=None):
     return Fn.BottleneckFunction.run(block, a, simt, out)
 
 
-def _bottleneck_body(block, a, simt=False, out=None):
+def _fusable_close(block, a, simt):
     ds = block.downsample
-    if (not simt and isinstance(ds, nn.Sequential) and len(ds) == 2 and _plain_1x1(ds[0]) and _plain_1x1(block.conv3)
+    return (not simt and isinstance(ds, nn.Sequential) and len(ds) == 2 and _plain_1x1(ds[0]) and _plain_1x1(block.conv3)
             and not ds[1].training and len(set(_conv_geometry(ds[0])[0])) == 1 and (a.T > 1 or _conv_geometry(ds[0])[0][0] == 1)
-            and isinstance(ds[0], nn.Conv3d)):
+            and isinstance(ds[0], nn.Conv3d))
+
+
+def _bottleneck_body(block, a, simt=False, out=None):
+    if _fusable_close(block, a, simt):
         h = conv_bn_act(block.conv1, block.bn1, a, relu=True)
         h = conv_bn_act(block.conv2, block.bn2, h, relu=True)
         return _fused_close_with_projection(block, a, h, out)
@@ -510,22 +514,41 @@ def _run_segment(units, x, N, clips, simt):
     return buf
 
 
-def run_trunk(model, x, simt=False):
+def run_trunk(model, x, simt=False, trainable_from=None):
+    """The trunk on ``x``.  ``trainable_from`` (1..4): the blocks of ``layer{trainable_from}..layer4`` run breadth-first
+    through ``TrainableBlockFunction`` (the depth-first plan only covers the frozen units before them), and the result is a
+    ``TrainAct`` that ``run_head`` pools differentiably."""
     units = _trunk_units(model)
+    cut = len(units)
+    if trainable_from is not None:
+        first = getattr(model, "layer%d" % trainable_from)[0]
+        cut = next(i for i, (_, m) in enumerate(units) if m is first)
+    frozen, trained = units[:cut], units[cut:]
     N = x.N if isinstance(x, Act) else x.shape[0]
     plan = [] if simt else dfs_plan()
     a, ui = x, 0
     for n_units, clips in plan:
-        seg = units[ui:ui + n_units]
+        seg = frozen[ui:ui + n_units]
         if not seg:
             break
         ui += len(seg)
         a = _run_segment(seg, a, N, clips, simt) if 0 < clips < N else _run_units(seg, a, simt)
-    return _run_units(units[ui:], a, simt) if ui < len(units) else a
+    if ui < len(frozen):
+        a = _run_units(frozen[ui:], a, simt)
+    if not trained:
+        return a
+    scale = Fn.GradScale()
+    for _, blk in trained:
+        a = Fn.TrainableBlockFunction.run(blk, a, scale)
+    return TrainAct(a, scale)
 
 
 def run_head(model, a, head):
     """avgpool -> view(B,-1) -> last_linear (torchvision_models.py:460-464).  Returns fp32 [N][classes]."""
+    if isinstance(a, TrainAct):
+        # fine-tuned trunk: fp32 pooled features (the same fp16 values as below) through a differentiable pool
+        pooled = Fn.PoolFunction.apply(a.data, Fn._geom(a), a.grad_scale)
+        return Fn.linear(pooled, head.weight, head.bias) if isinstance(head, nn.Linear) else head(pooled)
     pooled = ops.avgpool_global(a)                     # fp16 [N][ld]
     if isinstance(head, nn.Linear) and torch.is_grad_enabled() and any(p.requires_grad for p in head.parameters()):
         # trainable head on frozen engine features: differentiable GEMM (functions.LinearFunction), same kernel
@@ -535,3 +558,141 @@ def run_head(model, a, head):
         return ops.linear(pooled, pl, out_f32=True)
     # user-swapped head (Identity, Dropout, custom module): hand it the pooled features like the reference does
     return head(pooled[:, :a.C].float())
+
+
+# ---------------------------------------------------------------------------------------------
+# fine-tuning: residual blocks with a backward, BatchNorm statistics frozen
+# ---------------------------------------------------------------------------------------------
+# Every layer is y = relu(z [+ r]) with z = s * conv(x, W) + shift, s = gamma / sqrt(var + eps), and the running statistics
+# fixed.  With gz = g_y * [y > 0] (b2_relu_grad_sum, which also sums gz per channel):
+#     dbeta  = sum gz
+#     dW     = s * R,                      R[k][c][tap] = sum_p gz[p][k] x[p*stride + tap - pad][c]   (b2_conv_ndhwc_wgrad)
+#     dgamma = (sum_{c,tap} W * R - mean * sum gz) / sqrt(var + eps)       (= sum gz * x_hat, without dividing by gamma)
+#     g_x    = conv(gz, flip(W * s)^T)                                      (the forward convolution kernels)
+# and the residual branch receives gz of the closing layer.  dgamma never divides by gamma, so a zero gamma (a zero-initialised
+# last BatchNorm of a block) gives exact gradients, and neither the pre-activation nor the residual has to be saved.
+# Gradients travel between blocks as fp16 scaled by one power of two per backward pass (a device scalar, GradScale); only the
+# fp32 parameter gradients are unscaled.
+class TrainAct(Act):
+    """The output Act of a fine-tuned trunk, carrying the GradScale its backward pass shares."""
+    __slots__ = ("grad_scale",)
+
+    def __init__(self, a, grad_scale):
+        super().__init__(a.data, a.N, a.T, a.H, a.W, a.C)
+        self.grad_scale = grad_scale
+
+
+def trainable_layers(block):
+    """[(conv, bn)] of a block in parameter order: conv1/bn1, conv2/bn2[, conv3/bn3][, type-B projection]."""
+    pairs = [(block.conv1, block.bn1), (block.conv2, block.bn2)]
+    if hasattr(block, "conv3"):
+        pairs.append((block.conv3, block.bn3))
+    if isinstance(block.downsample, nn.Sequential):
+        pairs.append((block.downsample[0], block.downsample[1]))
+    return pairs
+
+
+def train_forward(block, a):
+    """The block's forward (the frozen body's kernels and results) and the activations its backward needs."""
+    if hasattr(block, "conv3"):
+        h1 = conv_bn_act(block.conv1, block.bn1, a, relu=True)
+        h2 = conv_bn_act(block.conv2, block.bn2, h1, relu=True)
+        if _fusable_close(block, a, False):
+            out = _fused_close_with_projection(block, a, h2)
+        else:
+            out = conv_bn_act(block.conv3, block.bn3, h2, residual=_shortcut(block, a, False), relu=True)
+        return out, (h1, h2)
+    h1 = conv_bn_act(block.conv1, block.bn1, a, relu=True)
+    return conv_bn_act(block.conv2, block.bn2, h1, residual=_shortcut(block, a, False), relu=True), (h1,)
+
+
+def _dgrad_filter(conv, bn, in_pitch):
+    """PackedConv of flip(W * s)^T: the stride-1 convolution of the (dilated) output gradient that gives the input gradient."""
+    def build():
+        s, _ = ops.fold_affine(conv.weight.shape[0], None, bn, conv.weight.device)
+        w = (conv.weight.detach().float() * s[:, None, None, None, None]).transpose(0, 1).flip(2, 3, 4).contiguous()
+        return ops.PackedConv(w, None, None, (1, 1, 1), _conv_geometry(conv)[1], in_pitch=in_pitch)
+    return _cached(conv, "dgrad", _sig(conv.weight, *_bn_tensors(bn)) + (in_pitch,), build)
+
+
+def _dgrad(conv, bn, gz, x_geom, residual=None):
+    """Input gradient of ``conv`` (x geometry (N, T, H, W, C)) from the masked output gradient ``gz``; ``residual`` (an Act of
+    the input geometry) is added in the epilogue."""
+    N, T, H, W, _ = x_geom
+    stride = _conv_geometry(conv)[0]
+    if stride != (1, 1, 1):
+        if len(set(stride)) != 1:
+            raise NotImplementedError("anisotropic strides have no data gradient here")
+        if tuple(conv.weight.shape[2:]) == (1, 1, 1):
+            raise ValueError("strided 1x1x1 data gradients go through strided_scatter_add_")
+        gz = ops.zero_dilate(gz, T, H, W, stride[0])
+    return ops.conv(gz, _dgrad_filter(conv, bn, gz.ld), residual=residual)
+
+
+def _layer_grads(conv, bn, x, gz, gsum, scale, need_w, need_bn):
+    """(dW, dgamma, dbeta) of one conv + frozen BN from its input Act ``x`` and the masked gradient ``gz`` (scaled by ``scale``)."""
+    if not (need_w or need_bn):
+        return None, None, None
+    K, Cin = conv.weight.shape[:2]
+    kt, kh, kw = conv.weight.shape[2:]
+    stride, padding = _conv_geometry(conv)
+    dev = gz.data.device
+    R = ops.conv_wgrad(x, gz, K, (kt, kh, kw), stride, padding)
+    R = R.view(K, kt, kh, kw, -1)[..., :Cin].permute(0, 4, 1, 2, 3)
+    s, _ = ops.fold_affine(K, None, bn, dev)
+    inv = torch.rsqrt(bn.running_var.detach().float() + bn.eps)
+    dw = (R * (s / scale)[:, None, None, None, None]).contiguous() if need_w else None
+    dg = db = None
+    if need_bn:
+        S = gsum[:K]
+        dg = inv * ((conv.weight.detach().float() * R).sum((1, 2, 3, 4)) - bn.running_mean.detach().float() * S) / scale
+        db = S / scale
+    return dw, dg, db
+
+
+def train_backward(block, x, acts, out, g, scale, need_x, need_params):
+    """Gradients of one block: (g_x Act or None, [dW, dgamma, dbeta per trainable_layers(block)]).  ``x``, ``acts``, ``out``: the
+    block's input, hidden activations and output (Acts); ``g``: fp16 gradient of ``out`` scaled by the device scalar ``scale``;
+    ``need_params``: one flag per parameter, in the order of the returned list."""
+    layers = trainable_layers(block)
+    need = [need_params[3 * i:3 * i + 3] for i in range(len(layers))]
+    grads = [None] * (3 * len(layers))
+
+    def mask(y, g2d):
+        gz, gsum = ops.relu_grad_sum(y.data, g2d)
+        return Act(gz, y.N, y.T, y.H, y.W, y.C), gsum
+
+    def record(i, xin, gz, gsum):
+        conv, bn = layers[i]
+        grads[3 * i:3 * i + 3] = _layer_grads(conv, bn, xin, gz, gsum, scale, need[i][0], need[i][1] or need[i][2])
+
+    gz = mask(out, g)                                      # closing layer; also the residual branch's gradient
+    close = gz
+    hidden = [x] + list(acts)                              # input of layer i is hidden[i]
+    for i in range(len(hidden) - 1, -1, -1):
+        record(i, hidden[i], *gz)
+        if i == 0:
+            break
+        conv, bn = layers[i]
+        gz = mask(hidden[i], _dgrad(conv, bn, gz[0], _geom_of(hidden[i])).data)
+    ds = block.downsample
+    sub = None
+    if isinstance(ds, nn.Sequential):
+        stride = _conv_geometry(ds[0])[0][0]
+        record(len(layers) - 1, x, *close)                # the patch gather subsamples x itself
+        sub = ops.conv(close[0], _dgrad_filter(ds[0], ds[1], close[0].ld)) if need_x else None
+    elif ds is not None:
+        stride, sub = ds.stride, close[0] if need_x else None
+    else:
+        stride, sub = 1, close[0] if need_x else None
+    if not need_x:
+        return None, grads
+    conv1, bn1 = layers[0]
+    gx = _dgrad(conv1, bn1, gz[0], _geom_of(x), residual=sub if stride == 1 else None)
+    if stride != 1:
+        ops.strided_scatter_add_(gx, sub.data, ops._round_up(x.C, 8), stride)
+    return gx, grads
+
+
+def _geom_of(a):
+    return (a.N, a.T, a.H, a.W, a.C)

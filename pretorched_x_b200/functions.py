@@ -13,6 +13,9 @@ Two kinds:
   torchvision_models.py:463-464) and, built from it, the TRN relation MLP (trn.py:39-49).  ``forward`` and both
   gradient products run on the same tcgen05 GEMM (``b2_gemm_f16``: fp16 operands, fp32 accumulation and output), so a
   head can be trained on engine features without leaving the library.
+* **Fine-tuned residual blocks** -- ``TrainableBlockFunction`` (resnet3d ``BasicBlock`` / ``Bottleneck`` of the stages
+  ``ResNet3D.enable_fine_tuning`` opens, frozen BatchNorm statistics) and ``PoolFunction`` (the global average in front of the
+  head) have a backward; their gradients travel in fp16 scaled by one power of two per backward pass (``GradScale``).
 
 Tensors cross a Function boundary as the raw ``[N*T*H*W][ld]`` fp16 matrix of an ``ops.Act`` plus its geometry tuple.
 ``out`` (optional, last argument of the block bodies): a preallocated ``[rows][ld]`` fp16 row range the body's LAST kernel writes
@@ -125,6 +128,84 @@ def _unit_affine(n, dev):
     return torch.ones(n, dtype=torch.float32, device=dev), torch.zeros(n, dtype=torch.float32, device=dev)
 
 
+# One power of two per backward pass, chosen so that the largest gradient entering fp16 lands in [2^7, 2^8): per-element
+# gradients of a mean-reduced loss sit near 1e-6 in the last stages, where fp16 has only subnormals left, and the headroom
+# below 65504 leaves room for gradients to grow through the trunk.
+_GRAD_TARGET = 2.0 ** 8
+
+
+def pow2_scale(amax):
+    """2^floor(log2(target / amax)) as an fp32 device scalar, 1 where amax is 0 or not finite; no host synchronisation."""
+    e = torch.floor(torch.log2(_GRAD_TARGET / amax.float())).clamp(-100.0, 100.0)
+    return torch.where(torch.isfinite(amax) & (amax > 0), torch.exp2(e), torch.ones_like(e))
+
+
+class GradScale:
+    """The gradient scale one backward pass of a fine-tuned trunk shares: set by ``PoolFunction.backward`` (where the gradient
+    enters the trunk) and read by every ``TrainableBlockFunction.backward`` after it."""
+    __slots__ = ("value",)
+
+    def __init__(self):
+        self.value = None
+
+    def get(self, dev):
+        return self.value if self.value is not None else torch.ones((), dtype=torch.float32, device=dev)
+
+
+class PoolFunction(torch.autograd.Function):
+    """Global average pool of a fine-tuned trunk's output -> fp32 [N][C] (exactly the fp16 values the frozen head pools).
+    Backward: the scaled fp16 gradient of every position, g / (T*H*W) * scale."""
+
+    @staticmethod
+    def forward(ctx, x2d, geom, grad_scale):
+        from .ops import avgpool_global
+        ctx.geom, ctx.ld, ctx.grad_scale = geom, x2d.shape[1], grad_scale
+        return avgpool_global(Act(x2d, *geom))[:, :geom[4]].float()
+
+    @staticmethod
+    def backward(ctx, g):
+        N, T, H, W, C = ctx.geom
+        P = T * H * W
+        g = g / P
+        s = pow2_scale(g.abs().amax())
+        ctx.grad_scale.value = s
+        gx = torch.zeros((N, P, ctx.ld), dtype=torch.float16, device=g.device)
+        gx[:, :, :C] = (g * s).to(torch.float16)[:, None, :]
+        return gx.view(N * P, ctx.ld), None, None
+
+
+class TrainableBlockFunction(torch.autograd.Function):
+    """A resnet3d BasicBlock / Bottleneck with a backward (frozen BatchNorm statistics; engine.train_backward).  The
+    parameters of ``engine.trainable_layers(block)`` (conv weight, BN weight, BN bias per layer) are inputs, so autograd
+    hands their gradients to them; the gradient of the output travels scaled by ``grad_scale``."""
+
+    @staticmethod
+    def forward(ctx, x2d, geom, block, grad_scale, *params):
+        from . import engine
+        x = Act(x2d, *geom)
+        out, acts = engine.train_forward(block, x)
+        ctx.block, ctx.grad_scale = block, grad_scale
+        ctx.geoms = [geom] + [_geom(h) for h in acts] + [_geom(out)]
+        ctx.save_for_backward(x2d, *[h.data for h in acts], out.data)
+        return out.data, _geom(out)
+
+    @staticmethod
+    def backward(ctx, g, _):
+        from . import engine
+        saved = ctx.saved_tensors
+        acts = [Act(t, *gm) for t, gm in zip(saved, ctx.geoms)]
+        gx, grads = engine.train_backward(ctx.block, acts[0], acts[1:-1], acts[-1], g.contiguous(), ctx.grad_scale.get(g.device),
+                                          ctx.needs_input_grad[0], ctx.needs_input_grad[4:])
+        return (gx.data if gx is not None else None, None, None, None) + tuple(grads)
+
+    @classmethod
+    def run(cls, block, a, grad_scale):
+        from . import engine
+        params = [t for conv, bn in engine.trainable_layers(block) for t in (conv.weight, bn.weight, bn.bias)]
+        data, geom = cls.apply(a.data, _geom(a), block, grad_scale, *params)
+        return Act(data, *geom)
+
+
 class LinearFunction(torch.autograd.Function):
     """y = x W^T + b on tcgen05 (fp16 operands, fp32 accumulate / output), with
     dL/dx = g W, dL/dW = g^T x, dL/db = sum_rows g computed by the same kernel (D = A . B^T with K-major operands:
@@ -150,18 +231,19 @@ class LinearFunction(torch.autograd.Function):
         rows, out_f = gy.shape
         in_f = ctx.in_features
         gx = gw = gb = None
-        g16 = _f16_padded(gy)                                            # [rows][out_p]
+        s = pow2_scale(gy.abs().amax())                                  # gy is cast to fp16 scaled, the fp32 products unscaled
+        g16 = _f16_padded(gy * s)                                        # [rows][out_p]
         if ctx.needs_input_grad[0]:
             wt = _f16_padded(weight.detach().t())                        # [in][out_p]: B operand, K = out
             one, zero = _unit_affine(in_f, dev)
-            gx = ops.gemm(g16, wt, one, zero, rows, in_f, out_f, out_f32=True)
+            gx = ops.gemm(g16, wt, one, zero, rows, in_f, out_f, out_f32=True) / s
             if ctx.relu_input:
                 gx = gx * (x16[:, :in_f] > 0)
         if ctx.needs_input_grad[1]:
-            gt = _f16_padded(gy.t())                                     # [out][rows_p]: A operand, K = rows
+            gt = _f16_padded((gy * s).t())                               # [out][rows_p]: A operand, K = rows
             xt = _f16_padded(x16[:, :in_f].t())                          # [in][rows_p]
             one, zero = _unit_affine(in_f, dev)
-            gw = ops.gemm(gt, xt, one, zero, out_f, in_f, rows, out_f32=True)
+            gw = ops.gemm(gt, xt, one, zero, out_f, in_f, rows, out_f32=True) / s
         if ctx.has_bias and ctx.needs_input_grad[2]:
             gb = gy.sum(0)
         return gx, gw, gb, None

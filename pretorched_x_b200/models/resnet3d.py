@@ -186,12 +186,33 @@ class ResNet3D(engine.CacheOwner, nn.Module):
             if src in state_dict and dst not in state_dict:
                 state_dict[dst] = state_dict.pop(src)
 
+    # -- fine-tuning -----------------------------------------------------------------------------
+    def enable_fine_tuning(self, ft_begin_index):
+        """Give ``layer{ft_begin_index}..layer4`` a backward (opt-in; returns the model).  While grad mode is on, their blocks run
+        through ``functions.TrainableBlockFunction``: conv weights and BatchNorm weight / bias receive ``.grad``, with the
+        BatchNorm running statistics frozen (the model stays in ``eval()``; ``train()`` still refuses to run).  Earlier stages
+        stay frozen.  5: head only (the default behaviour); ``None``: off.  Only ``resnet3d.BasicBlock`` / ``Bottleneck`` with
+        plain ``nn.Conv3d`` convolutions have a backward; the stem (0) has none."""
+        if ft_begin_index is None or ft_begin_index == 5:
+            self._b2_ft_begin = None
+            return self
+        if ft_begin_index == 0:
+            raise NotImplementedError("the stem (conv1 / bn1) has no backward: fine-tuning starts at layer1 or later")
+        if ft_begin_index not in (1, 2, 3, 4):
+            raise ValueError("ft_begin_index must be 0..5 or None, got %r" % (ft_begin_index,))
+        for i in range(ft_begin_index, 5):
+            for blk in getattr(self, "layer%d" % i):
+                _check_trainable(blk, "layer%d" % i)
+        self._b2_ft_begin = int(ft_begin_index)
+        return self
+
     # -- reference API ------------------------------------------------------------------------
     def features_act(self, x):
         """Trunk on the engine's native layout (fp16 NDHWC ``Act``)."""
         if self.training:
             raise RuntimeError("the forward engine is inference-only: call model.eval() first")
-        return engine.run_trunk(self, x)
+        ft = self.__dict__.get("_b2_ft_begin")
+        return engine.run_trunk(self, x, trainable_from=ft if torch.is_grad_enabled() else None)
 
     def features(self, input):
         return ops.to_ncdhw(self.features_act(input))
@@ -202,6 +223,41 @@ class ResNet3D(engine.CacheOwner, nn.Module):
 
     def forward(self, input):
         return self.logits(self.features_act(input))
+
+
+def _check_trainable(blk, where):
+    """Raise NotImplementedError unless ``blk`` is a block the fine-tuning backward covers (exact types: the R(2+1)D blocks
+    subclass these)."""
+    ok = type(blk) in (BasicBlock, Bottleneck) and getattr(blk, "nonlocalblock", None) is None
+    convs = [blk.conv1, blk.conv2] + ([blk.conv3] if hasattr(blk, "conv3") else [])
+    ds = blk.downsample
+    if isinstance(ds, nn.Sequential):
+        ok = ok and len(ds) == 2 and isinstance(ds[1], nn.BatchNorm3d)
+        convs.append(ds[0])
+    else:
+        ok = ok and (ds is None or isinstance(ds, ShortcutA))
+    ok = ok and all(type(c) is nn.Conv3d and c.bias is None and c.groups == 1 and tuple(c.dilation) == (1, 1, 1)
+                    and len(set(c.stride)) == 1 for c in convs)
+    if not ok:
+        raise NotImplementedError("%s: %s blocks have no backward (fine-tuning covers resnet3d BasicBlock / Bottleneck with "
+                                  "plain Conv3d convolutions)" % (where, type(blk).__name__))
+
+
+def get_fine_tuning_parameters(model, ft_begin_index):
+    """Optimizer parameter groups that train ``layer{ft_begin_index}..layer4`` and the head, with lr 0 for everything else
+    (resnet3D.py:221-239).  ``ft_begin_index == 0``: ``model.parameters()``.  The head is matched by the model's
+    ``head_name`` (``last_linear``, or ``fc``).  Changes no model state; pair it with ``model.enable_fine_tuning``."""
+    if ft_begin_index == 0:
+        return model.parameters()
+    ft_module_names = ['layer{}'.format(i) for i in range(ft_begin_index, 5)]
+    ft_module_names.append(getattr(model, 'head_name', 'fc'))
+    parameters = []
+    for k, v in model.named_parameters():
+        if any(name in k for name in ft_module_names):
+            parameters.append({'params': v})
+        else:
+            parameters.append({'params': v, 'lr': 0.0})
+    return parameters
 
 
 def _attach_settings(model, settings):

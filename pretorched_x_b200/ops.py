@@ -589,3 +589,73 @@ def rgb_head(partial, bias, N, H, W, K=3, out_dtype=torch.float32, out=None):
         _lib.check(_lib.load().b2_rgb_head_gather_tanh(_ptr(partial), partial.stride(0), _ptr(bias), _ptr(y), N, H, W, K,
                                                       int(out_dtype == torch.float32), _stream()), "b2_rgb_head_gather_tanh")
     return y
+
+
+# ---------------------------------------------------------------------------------------------
+# backward of the residual blocks (frozen BatchNorm statistics): see engine.py, "fine-tuning"
+# ---------------------------------------------------------------------------------------------
+@_on_device
+def relu_grad_sum(y2d, g2d):
+    """ReLU backward: ``(gz, s)`` with gz = g * [y > 0] (fp16, y's shape) and s[c] = sum over rows of gz[:, c] (fp32 [ld]),
+    reduced in a fixed order.  y2d: fp16 [M][ld] (a ReLU output), g2d: fp16 [M][>= ld]."""
+    M, ld = y2d.shape
+    if g2d.shape[0] != M or g2d.shape[1] < ld or g2d.stride(1) != 1 or y2d.stride(0) != ld:
+        raise ValueError("gradient %s does not match activation %s" % (tuple(g2d.shape), tuple(y2d.shape)))
+    lib = _lib.load()
+    gz = torch.empty_like(y2d)
+    partial = torch.empty((lib.b2_relu_grad_sum_partials(M, ld), ld), dtype=torch.float32, device=y2d.device)
+    s = torch.empty(ld, dtype=torch.float32, device=y2d.device)
+    with _timed("bwd_eltwise", "relu_grad_sum C%d M=%d" % (ld, M), 0.0, 6.0 * M * ld):
+        _lib.check(lib.b2_relu_grad_sum(_ptr(y2d), ld, _ptr(g2d), g2d.stride(0), _ptr(gz), M, _ptr(partial), _ptr(s), _stream()),
+                   "b2_relu_grad_sum")
+    return gz, s
+
+
+def wgrad_args(x, g, K, kernel, stride, padding, dw=None, work=None):
+    """WgradArgs for the weight gradient of a convolution with input Act ``x`` and output gradient Act ``g`` (K filters)."""
+    from ._lib import WgradArgs
+    a = WgradArgs()
+    a.x, a.g, a.dw, a.work = _ptr(x.data), _ptr(g.data), _ptr(dw), _ptr(work)
+    a.N, a.T, a.H, a.W, a.ldx, a.C = x.N, x.T, x.H, x.W, x.ld, _round_up(x.C, 8)
+    a.ldg, a.K = g.ld, K
+    (a.kt, a.kh, a.kw), (a.st, a.sh, a.sw), (a.pt, a.ph, a.pw) = kernel, stride, padding
+    return a
+
+
+@_on_device
+def conv_wgrad(x, g, K, kernel, stride, padding):
+    """Weight gradient sum_p g[p][k] x[p*stride + tap - pad][c] on tcgen05 (b2_conv_ndhwc_wgrad): fp32 [K][taps][C]."""
+    taps = kernel[0] * kernel[1] * kernel[2]
+    C = _round_up(x.C, 8)
+    dw = torch.empty((K, taps, C), dtype=torch.float32, device=x.data.device)
+    lib = _lib.load()
+    args = wgrad_args(x, g, K, kernel, stride, padding, dw)
+    n = lib.b2_wgrad_workspace_floats(ctypes.byref(args))
+    work = torch.empty(n, dtype=torch.float32, device=x.data.device) if n else None
+    args.work = _ptr(work)
+    P = g.N * g.T * g.H * g.W
+    with _timed("wgrad", "wgrad %dx%dx%d C%d->%d P=%d" % (kernel + (C, K, P)), 2.0 * P * K * C * taps,
+                2.0 * (x.M * x.ld * taps + g.M * g.ld) + 4.0 * dw.numel() * (1 + 2 * (n > 0))):
+        _lib.check(lib.b2_conv_ndhwc_wgrad(ctypes.byref(args), _stream()), "b2_conv_ndhwc_wgrad")
+    return dw
+
+
+@_on_device
+def zero_dilate(g, T, H, W, stride):
+    """Act g of a stride-``stride`` output -> Act of the input geometry (T, H, W) holding g at the strided positions, 0 elsewhere."""
+    y = torch.empty((g.N * T * H * W, g.ld), dtype=torch.float16, device=g.data.device)
+    with _timed("bwd_eltwise", "zero_dilate C%d M=%d" % (g.C, y.shape[0]), 0.0, 2.0 * (g.M + y.shape[0]) * g.ld):
+        _lib.check(_lib.load().b2_zero_dilate_scatter(_ptr(g.data), _ptr(y), g.N, T, H, W, g.ld, stride, _stream()),
+                   "b2_zero_dilate_scatter")
+    return Act(y, g.N, T, H, W, g.C)
+
+
+@_on_device
+def strided_scatter_add_(y, g2d, C, stride):
+    """In place: y[n, s*t, s*h, s*w, :C] += g2d[(n, t, h, w), :C] (the data gradient of a stride-s subsampling)."""
+    if g2d.shape[0] != y.N * ((y.T - 1) // stride + 1) * ((y.H - 1) // stride + 1) * ((y.W - 1) // stride + 1):
+        raise ValueError("subsampled gradient rows %d do not match %r at stride %d" % (g2d.shape[0], y, stride))
+    with _timed("bwd_eltwise", "strided_scatter_add C%d M=%d" % (C, g2d.shape[0]), 0.0, 6.0 * g2d.shape[0] * C):
+        _lib.check(_lib.load().b2_strided_scatter_add(_ptr(g2d), g2d.stride(0), _ptr(y.data), y.ld, y.N, y.T, y.H, y.W, C, stride,
+                                                     _stream()), "b2_strided_scatter_add")
+    return y
